@@ -19,6 +19,8 @@ The same JSON line (rank 0, stdout) carries a `configs` block with the other SUR
   config4  the 96-sample plate at 5,000x, samples round-robin over the N ranks, no communication (strong scaling)
 and `e2e_api`: LiveVariantCaller.process_bam(BAM on disk) + prepare_variants() (N = 1).
 `--legs main` runs the headline workload only (kernel experiments).
+`--dump-outputs DIR` writes what the last timed step computed as .npy files, so that two builds can be compared output
+for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -27,11 +29,13 @@ import ctypes
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "covid-spings-variant-caller_b200")
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
 for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
@@ -51,9 +55,10 @@ def log(*a):
 
 
 # ------------------------------------------------------------------------------------------------ workloads
-def _cached(cache: str, make):
-    """(ref, ReadBatch) cached under /tmp so the arms of one box do not regenerate it."""
+def _cached(name: str, make):
+    """(ref, ReadBatch) cached in the temporary directory so the arms of one machine do not regenerate it."""
     from lvc_b200 import packing
+    cache = os.path.join(tempfile.gettempdir(), name)
     if os.path.exists(cache):
         try:
             z = np.load(cache)
@@ -74,7 +79,7 @@ def _cached(cache: str, make):
 
 def make_workload(seed: int, n_pairs: int):
     from lvc_b200 import synth
-    return _cached(f"/tmp/lvc_bench_cfg2_{seed}_{n_pairs}.npz", lambda: synth.amplicon_sample(seed=seed, n_pairs=n_pairs))
+    return _cached(f"lvc_bench_cfg2_{seed}_{n_pairs}.npz", lambda: synth.amplicon_sample(seed=seed, n_pairs=n_pairs))
 
 
 def live_bytes(batch) -> int:
@@ -352,7 +357,7 @@ def leg_config3(torch, capi, records, stream, dev, distinct=4, n_batches=100):
 
 def config5_workload(ref_len=1_000_000):
     from lvc_b200 import synth
-    return _cached(f"/tmp/lvc_bench_cfg5_{ref_len}.npz",
+    return _cached(f"lvc_bench_cfg5_{ref_len}.npz",
                    lambda: synth.shotgun_sample(ref_len=ref_len, n_snvs=max(10, ref_len // 10000))[:2])
 
 
@@ -517,7 +522,7 @@ def leg_config4(torch, dist, capi, records, stream, dev, world, rank, n_samples=
     mine = ldist.assign_samples(n_samples, world, rank)
     gen = mine[:max(1, min(distinct, len(mine)))]
     t0 = time.time()
-    data = [_cached(f"/tmp/lvc_bench_cfg4_{20260300 + s}.npz",
+    data = [_cached(f"lvc_bench_cfg4_{20260300 + s}.npz",
                     lambda s=s: synth.amplicon_sample(seed=20260300 + s, n_pairs=N_PAIRS // 2)) for s in gen]
     data = [(r, in_form(b)) for r, b in data]
     gen_s = time.time() - t0
@@ -574,13 +579,12 @@ def leg_config4(torch, dist, capi, records, stream, dev, world, rank, n_samples=
                       "neighbouring kernels); CUDA events, max over ranks"}
 
 
-def leg_e2e_api(torch, ref, batch, stream, local, reps=3):
+def leg_e2e_api(torch, ref, batch, stream, local, tmp, reps=3):
     """The call the reference's server makes (client_server/vc_queue.py:142-144): process_bam(BAM on disk) +
-    prepare_variants(), BAM decode, admission and mate-overlap pass included."""
+    prepare_variants(), BAM decode, admission and mate-overlap pass included.  The BAM is written to directory `tmp`."""
     from lvc_b200 import samio, synth
     from variant_caller.live_variant_caller import LiveVariantCaller
-    bam = f"/tmp/lvc_bench_cfg2_{os.getpid()}.bam"
-    fasta = f"/tmp/lvc_bench_api_{os.getpid()}.fasta"
+    bam, fasta = os.path.join(tmp, "cfg2.bam"), os.path.join(tmp, "ref.fasta")
     t0 = time.time()
     ids, mpos, tlen = synth.amplicon_pairing(batch, N_PAIRS, len(ref))
     samio.write_bam_batch(bam, ("NC_045512.2", len(ref)), batch, name_id=ids, mate_pos=mpos, tlen=tlen)
@@ -606,15 +610,25 @@ def leg_e2e_api(torch, ref, batch, stream, local, reps=3):
     dt = (time.perf_counter() - t1) / reps
     size = os.path.getsize(bam)
     lvc.close()
-    for p in (bam, fasta):
-        try:
-            os.remove(p)
-        except OSError:
-            pass
     return {"api": "LiveVariantCaller.process_bam(BAM on disk) + prepare_variants()", "value": batch.aligned_bases() / dt,
             "unit": UNIT, "ms_per_step": dt * 1e3, "ingest_ms": min(t_ing) * 1e3, "bam_bytes": size, "reads": n_reads,
             "mate_pairs_rewritten": pairs, "variants": len(variants), "steps": reps, "host_threads": os.cpu_count(),
             "bam_write_s": round(write_s, 1), "timing": "host wall clock around the calls (the path is host bound)"}
+
+
+def dump_outputs(h, out_dir: str) -> None:
+    """What the caller of the timed step receives after its last step, as float64 .npy files in `out_dir` (2.2 MB for
+    config 2): the candidate records of lvc_fetch_candidates, one array per field, sorted by position and allele (the
+    kernel appends them through an atomic counter, in no fixed order), and the dense per-position outputs of the genotype pass (lvc_copy_dense:
+    depth, allele depths and likelihoods of the four allele slots)."""
+    h.check_async()
+    cand = np.sort(h.fetch_candidates(), order=["pos", "code"])
+    depth, ad, lik = h.copy_dense()
+    arrays = {f"candidates_{k}": cand[k] for k in ("pos", "code", "ref", "ad", "dp", "first", "L", "S", "esum")}
+    arrays.update(depth=depth, allele_depth=ad, likelihood=lik)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ main
@@ -638,6 +652,9 @@ def main():
                          "(what process_bam does; 0.5 payload bytes per base over PCIe); nibbles: 4-bit BAM codes (0.75)")
     ap.add_argument("--quality-form", default="codes", choices=["codes", "bytes"],
                     help="codes: batches whose qualities take <= 4 values ship 2-bit codes (what process_bam does); bytes: one phred byte per base")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them computed to DIR/<name>.npy (rank 0; the "
+                         "tables accumulate over the warm-up and timed steps, so equal arguments give equal outputs)")
     args = ap.parse_args()
     global QUALITY_FORM
     QUALITY_FORM = args.quality_form
@@ -722,6 +739,8 @@ def main():
     sampler.start()
     # (1) the step time: EXACTLY --steps steps, the two kernels of a step back to back, nothing else on the stream
     ms, launches = timed_region(args.steps, False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(h, args.dump_outputs)
     # (2) the same steps again with per-kernel events: the kernels' own durations for the roofline
     ms_ev, _ = timed_region(args.steps, True)
     tile_ms, tile_n = h.get_timing(0)
@@ -739,11 +758,12 @@ def main():
     value = world * bases * args.steps / (ms * 1e-3)
 
     # ---- end to end through the public API: pinned host SoA -> process_batch -> prepare_variants
-    fasta = f"/tmp/lvc_bench_ref_{rank}.fasta"
-    with open(fasta, "w") as fh:
-        fh.write(">NC_045512.2\n" + ref + "\n")
-    lvc = LiveVariantCaller(fasta, THRESH["minBQ"], THRESH["minMQ"], THRESH["minDP"], THRESH["minAD"], THRESH["ratio"], 1,
-                            device=local)
+    with tempfile.TemporaryDirectory(prefix="lvc_bench_") as tmp:
+        fasta = os.path.join(tmp, "ref.fasta")
+        with open(fasta, "w") as fh:
+            fh.write(">NC_045512.2\n" + ref + "\n")
+        lvc = LiveVariantCaller(fasta, THRESH["minBQ"], THRESH["minMQ"], THRESH["minDP"], THRESH["minAD"], THRESH["ratio"],
+                                1, device=local)
     lvc._handle.set_stream(stream.cuda_stream)
     lvc._handle.set_impl(args.kernel_impl)
 
@@ -830,7 +850,8 @@ def main():
     if "config3" in legs and world == 1:
         configs["config3"] = guarded("config3", lambda: leg_config3(torch, capi, records, stream, dev))
     if "e2e_api" in legs and world == 1:
-        e2e_api = guarded("e2e_api", lambda: leg_e2e_api(torch, ref, batch, stream, local))
+        with tempfile.TemporaryDirectory(prefix="lvc_bench_") as tmp:
+            e2e_api = guarded("e2e_api", lambda: leg_e2e_api(torch, ref, batch, stream, local, tmp))
 
     if rank == 0:
         peak, peak_src = measured_peak_gbs()

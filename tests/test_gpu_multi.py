@@ -19,7 +19,7 @@ def _free_port():
     return p
 
 
-def _worker(rank, world, port, rows, ref, q, mode="full"):
+def _worker(rank, world, port, rows, ref, q, workdir, mode="full"):
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     for p in (root, os.path.join(root, "covid-spings-variant-caller_b200"), os.path.join(root, "tests")):
@@ -33,7 +33,7 @@ def _worker(rank, world, port, rows, ref, q, mode="full"):
     torch.cuda.set_device(rank)
     dist.init_process_group("nccl", init_method=f"tcp://127.0.0.1:{port}", rank=rank, world_size=world,
                             device_id=torch.device("cuda", rank))
-    fa = f"/tmp/lvc_multi_{rank}.fasta"
+    fa = os.path.join(workdir, f"rank{rank}.fasta")
     with open(fa, "w") as fh:
         fh.write(">c\n" + ref + "\n")
     th = dict(minBQ=13, minMQ=0, minDP=3, minAD=2, ratio=0.05)
@@ -94,7 +94,7 @@ def test_two_ranks_equal_one(lib, golden_synth, tmp_path):
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, rows, ref, q)) for r in range(2)]
+    procs = [ctx.Process(target=_worker, args=(r, 2, port, rows, ref, q, str(tmp_path))) for r in range(2)]
     for p in procs:
         p.start()
     out, mem = q.get(timeout=300)
@@ -128,7 +128,7 @@ def test_two_ranks_halo_exchange_equal_one(lib, golden_synth, tmp_path):
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, rows, ref, q, "halo")) for r in range(2)]
+    procs = [ctx.Process(target=_worker, args=(r, 2, port, rows, ref, q, str(tmp_path), "halo")) for r in range(2)]
     for p in procs:
         p.start()
     out, slices = q.get(timeout=300)
@@ -169,7 +169,7 @@ def test_two_ranks_library_exchange_equal_one(lib, golden_synth, tmp_path, mode)
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, rows, ref, q, mode)) for r in range(2)]
+    procs = [ctx.Process(target=_worker, args=(r, 2, port, rows, ref, q, str(tmp_path), mode)) for r in range(2)]
     for p in procs:
         p.start()
     out, res = q.get(timeout=300)

@@ -1,9 +1,9 @@
 """Cross-check against the REAL reference wherever pysam can be imported (SURVEY 8d(2), Appendix B checklist).
 
 The pileup half of the oracle (CIGAR walk, deletion-entry quality rule, max_depth admission, mate overlaps) restates
-htslib, which is neither in /root/reference nor in this image, so it is "parity unpinned" (oracle/pileup_oracle.py
-header).  This module is the pin: when `import pysam` succeeds AND the reference tree is reachable (LVC_REFERENCE,
-baseline/_ref, /root/reference), it writes BAMs with samio.write_bam, runs the UNMODIFIED
+htslib, which is neither in the reference project nor a dependency of this one, so it is "parity unpinned"
+(oracle/pileup_oracle.py header).  This module is the pin: when `import pysam` succeeds AND the environment variable
+LVC_REFERENCE names a checkout of the reference project, it writes BAMs with samio.write_bam, runs the UNMODIFIED
 variant_caller/live_variant_caller.py:21 `LiveVariantCaller` (process_bam :54-72, prepare_variants :120-231) on them
 and compares `memory` and the records with the oracle (no GPU needed) and with the drop-in class (GPU).  When the
 import fails it says so -- with the reason -- so that the test log of every box records the pysam / htslib status.
@@ -20,7 +20,7 @@ import numpy as np
 import pytest
 
 from oracle import pileup_oracle as po
-from conftest import GOLD, ROOT
+from conftest import GOLD
 
 
 def _pysam_status():
@@ -35,9 +35,9 @@ def _pysam_status():
 
 
 def _reference_tree():
-    for cand in (os.environ.get("LVC_REFERENCE"), os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if cand and os.path.exists(os.path.join(cand, "variant_caller", "live_variant_caller.py")):
-            return cand
+    cand = os.environ.get("LVC_REFERENCE")
+    if cand and os.path.exists(os.path.join(cand, "variant_caller", "live_variant_caller.py")):
+        return cand
     return None
 
 

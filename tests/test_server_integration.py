@@ -1,10 +1,9 @@
 """Server integration (SURVEY 8f-3): the reference's UNTOUCHED task queue drives the drop-in class.
 
 `client_server/vc_queue.py:123-146` (`VCQueue._process_bam`: samtools sort + index -> load_checkpoint -> process_bam ->
-create_checkpoint -> write_vcf) is imported from an unmodified copy of the reference tree (LVC_REFERENCE,
-baseline/_ref -- where __graft_entry__.build() mirrors /root/reference when it is present -- or /root/reference),
-with the drop-in `variant_caller` package on the path instead of the reference's, exactly what a deployment that
-switches to this repo does.  pysam is not installable here, so `pysam.sort` / `pysam.index` are stubbed (the
+create_checkpoint -> write_vcf) is imported from an unmodified checkout of the reference project named by the
+LVC_REFERENCE environment variable (the test skips without one), with the drop-in `variant_caller` package on the
+path instead of the reference's, exactly what a deployment that switches to this repo does.  pysam is not installable here, so `pysam.sort` / `pysam.index` are stubbed (the
 drop-in sorts SAM input itself and needs no index).  The queue is fed like the reference's own test
 (test/vc_queue_test.py:30-36: put(('process', 'testdata/testfile.sam')); process()), and the VCF and the checkpoint
 it leaves on disk are compared with the oracle's.  Needs a GPU (the drop-in has no CPU path)."""
@@ -19,15 +18,15 @@ import types
 import pytest
 
 from oracle import pileup_oracle as po
-from conftest import GOLD, ROOT, PKG
+from conftest import GOLD, PKG
 
 pytestmark = pytest.mark.gpu
 
 
 def _reference_tree():
-    for cand in (os.environ.get("LVC_REFERENCE"), os.path.join(ROOT, "baseline", "_ref"), "/root/reference"):
-        if cand and os.path.exists(os.path.join(cand, "client_server", "vc_queue.py")):
-            return cand
+    cand = os.environ.get("LVC_REFERENCE")
+    if cand and os.path.exists(os.path.join(cand, "client_server", "vc_queue.py")):
+        return cand
     return None
 
 
@@ -40,7 +39,7 @@ def _norm(mem):
 def test_vcqueue_process_with_dropin(lib, tmp_path, monkeypatch, relaxed):
     tree = _reference_tree()
     if tree is None:
-        pytest.skip("no reference tree on this box (LVC_REFERENCE / baseline/_ref / /root/reference)")
+        pytest.skip("LVC_REFERENCE does not name a checkout of the reference project")
     work = tmp_path / "server"
     work.mkdir()
     for sub in ("client_server", "config_util"):                       # unmodified copies in a scratch directory
