@@ -19,6 +19,7 @@
 #include "deposit_tile5.cuh"
 #include "deposit_ont.cuh"
 #include "genotype.cuh"
+#include "consensus.cuh"
 #include "overlap.hpp"
 #include "qcode.hpp"
 
@@ -109,9 +110,14 @@ struct lvc_handle {
     double lut_host[512];                    // last uploaded e / 1-e tables
     bool lut_valid = false;
 
+    // consensus (lvc_consensus): its own ordered plane list, output letters and counters
+    DevBuf c_order_ptrs, c_seq, c_stats;
+    size_t cons_planes_uploaded = (size_t)-1;
+    int cons_grp_begin[5] = {0, 0, 0, 0, 0};
+
     // optional per-kernel timing (CUDA events on the launching stream)
     bool timing = false;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[3];   // 0 tiled deposit, 1 general deposit, 2 genotype
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[4];   // 0 tiled deposit, 1 general deposit, 2 genotype, 3 consensus
     std::vector<cudaEvent_t> ev_pool;
 };
 
@@ -304,12 +310,13 @@ void lvc_destroy(lvc_handle* h) {
     cudaFree(h->d_first_arr); cudaFree(h->d_newkeys); cudaFree(h->d_replay); cudaFree(h->d_status); cudaFree(h->d_keymap);
     if (h->h_status) cudaFreeHost(h->h_status);
     if (h->h_sample) cudaFreeHost(h->h_sample);
-    for (int w = 0; w < 3; ++w) for (auto& pr : h->ev[w]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
+    for (int w = 0; w < 4; ++w) for (auto& pr : h->ev[w]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
     for (auto e : h->ev_pool) cudaEventDestroy(e);
     cudaFree(h->d_elut); cudaFree(h->d_out_depth); cudaFree(h->d_out_ad); cudaFree(h->d_out_lik);
     cudaFree(h->d_cand_count);
     for (DevBuf* b : {&h->b_pos, &h->b_flag, &h->b_mapq, &h->b_keep, &h->b_coff, &h->b_cig, &h->b_soff, &h->b_seq,
-                      &h->b_qual, &h->g_order_ptrs, &h->g_order_keys, &h->g_cand, &h->g_pconst})
+                      &h->b_qual, &h->g_order_ptrs, &h->g_order_keys, &h->g_cand, &h->g_pconst, &h->c_order_ptrs,
+                      &h->c_seq, &h->c_stats})
         cudaFree(b->p);
     if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -839,7 +846,7 @@ int lvc_set_timing(lvc_handle* h, int on) {
 }
 
 int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launches) {
-    if (!h || which < 0 || which > 2 || !ms_total || !n_launches) return LVC_EINVAL;
+    if (!h || which < 0 || which > 3 || !ms_total || !n_launches) return LVC_EINVAL;
     CU(cudaSetDevice(h->device));
     CU(cudaStreamSynchronize(h->stream));
     double tot = 0.0;
@@ -1047,6 +1054,80 @@ int lvc_copy_dense(lvc_handle* h, uint32_t* depth, uint32_t* ad, double* lik) {
     if (ad) CU(cudaMemcpyAsync(ad, h->d_out_ad, G * 16, cudaMemcpyDeviceToHost, h->stream));
     if (lik) CU(cudaMemcpyAsync(lik, h->d_out_lik, G * 32, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
+    return LVC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// consensus + coverage statistics
+// ------------------------------------------------------------------------------------------------
+int lvc_consensus(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, double threshold,
+                  const uint32_t* depth_thresholds, int n_thresholds, uint8_t* seq_out, lvc_consensus_stats* stats_out) {
+    NvtxRange nvtx_range("lvc_consensus");
+    if (!h) return LVC_EINVAL;
+    if (!(threshold >= 0.0 && threshold <= 1.0))
+        return fail(h, LVC_EINVAL, "consensus threshold %g outside [0, 1]", threshold);
+    if (n_thresholds < 0 || n_thresholds > kConsMaxThr || (n_thresholds > 0 && !depth_thresholds))
+        return fail(h, LVC_EINVAL, "consensus: %d depth thresholds (0..%d)", n_thresholds, kConsMaxThr);
+    if (p1 < 0) { p0 = 0; p1 = h->G; }
+    if (p0 < 0 || p1 > h->G || p0 > p1)
+        return fail(h, LVC_EINVAL, "consensus range [%lld, %lld) outside [0, %lld)", (long long)p0, (long long)p1,
+                    (long long)h->G);
+    CU(cudaSetDevice(h->device));
+    const int np = (int)h->planes.size();
+    if (h->cons_planes_uploaded != (size_t)np) {     // planes are only ever appended: the count identifies the set
+        // order planes: group 0 first, then groups 1..3 (the genotype pass keeps its own list)
+        std::vector<int> order(np);
+        for (int i = 0; i < np; ++i) order[i] = i;
+        std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return h->plane_key[a] < h->plane_key[b]; });
+        std::vector<uint32_t*> ptrs(std::max(np, 1));
+        int grp_begin[5] = {0, 0, 0, 0, 0};
+        for (int i = 0; i < np; ++i) {
+            ptrs[i] = h->planes[order[i]];
+            grp_begin[(h->plane_key[order[i]] >> 8) + 1] = i + 1;
+        }
+        for (int g = 1; g <= 4; ++g) grp_begin[g] = std::max(grp_begin[g], grp_begin[g - 1]);
+        int rc = ensure(h, h->c_order_ptrs, ptrs.size() * sizeof(uint32_t*));
+        if (rc) return rc;
+        CU(cudaMemcpyAsync(h->c_order_ptrs.p, ptrs.data(), ptrs.size() * sizeof(uint32_t*), cudaMemcpyHostToDevice, h->stream));
+        CU(cudaStreamSynchronize(h->stream));             // `ptrs` goes out of scope
+        memcpy(h->cons_grp_begin, grp_begin, sizeof grp_begin);
+        h->cons_planes_uploaded = (size_t)np;
+    }
+    const int64_t n = p1 - p0;
+    int rc = ensure(h, h->c_seq, (size_t)std::max<int64_t>(n, 1));
+    if (rc) return rc;
+    rc = ensure(h, h->c_stats, CS_WORDS * sizeof(uint64_t));
+    if (rc) return rc;
+    CU(cudaMemsetAsync(h->c_stats.p, 0, CS_WORDS * sizeof(uint64_t), h->stream));
+    if (n > 0) {
+        ConsParams cp;
+        cp.p0 = p0; cp.p1 = p1; cp.min_depth = min_depth; cp.threshold = threshold;
+        for (int g = 0; g < 5; ++g) cp.grp_begin[g] = h->cons_grp_begin[g];
+        cp.n_thr = n_thresholds;
+        for (int i = 0; i < kConsMaxThr; ++i) cp.thr[i] = i < n_thresholds ? depth_thresholds[i] : 0u;
+        // a grid-stride loop over the range: a few blocks per SM keep enough rows in flight, and the block totals end in
+        // one atomic per counter per block
+        const unsigned blocks = (unsigned)std::min<int64_t>((n + kConsThreads - 1) / kConsThreads, (int64_t)h->sm_count * 16);
+        // launched without programmatic serialization: it starts after every earlier kernel of the stream has finished
+        KernelTimer t(h, 3);
+        k_consensus<<<blocks, kConsThreads, 0, h->stream>>>(cp, (const uint32_t* const*)h->c_order_ptrs.p, h->d_dels, h->d_ref,
+                                                             (uint8_t*)h->c_seq.p, (unsigned long long*)h->c_stats.p);
+        h->launches++;
+        CU(cudaGetLastError());
+    }
+    if (seq_out && n > 0) CU(cudaMemcpyAsync(seq_out, h->c_seq.p, (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+    uint64_t st[CS_WORDS];
+    CU(cudaMemcpyAsync(st, h->c_stats.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    if (stats_out) {
+        lvc_consensus_stats s;
+        memset(&s, 0, sizeof s);
+        s.n_positions = st[CS_POSITIONS]; s.depth_sum = st[CS_DEPTH_SUM]; s.depth_max = st[CS_DEPTH_MAX];
+        s.n_low_depth = st[CS_LOW_DEPTH]; s.n_N = st[CS_N]; s.n_deleted = st[CS_DELETED];
+        s.n_ambiguous = st[CS_AMBIGUOUS]; s.n_mismatch = st[CS_MISMATCH];
+        for (int i = 0; i < n_thresholds; ++i) s.depth_ge[i] = st[CS_GE + i];
+        *stats_out = s;
+    }
     return LVC_OK;
 }
 

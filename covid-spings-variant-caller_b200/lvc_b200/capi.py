@@ -50,6 +50,16 @@ CANDIDATE_DTYPE = np.dtype([("pos", "<i4"), ("code", "u1"), ("ref", "u1"), ("pad
                             ("esum", "<f8")])
 assert CANDIDATE_DTYPE.itemsize == C.sizeof(Candidate) == 48
 
+CONSENSUS_COUNTERS = ("n_positions", "depth_sum", "depth_max", "n_low_depth", "n_N", "n_deleted", "n_ambiguous",
+                      "n_mismatch")
+
+
+class ConsensusStats(C.Structure):
+    _fields_ = [(name, C.c_uint64) for name in CONSENSUS_COUNTERS] + [("depth_ge", C.c_uint64 * 8)]
+
+
+assert C.sizeof(ConsensusStats) == 128
+
 _lib: Optional[C.CDLL] = None
 
 # every symbol include/lvc.h declares: (name, restype, argtypes)
@@ -98,6 +108,8 @@ SIGNATURES = [
     ("lvc_fetch_candidates", C.c_int, [_H, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]),
     ("lvc_set_genotype_range", C.c_int, [_H, C.c_int64, C.c_int64]),
     ("lvc_copy_dense", C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p]),
+    ("lvc_consensus", C.c_int, [_H, C.c_int64, C.c_int64, C.c_uint64, C.c_double, C.c_void_p, C.c_int, C.c_void_p,
+                                C.POINTER(ConsensusStats)]),
     ("lvc_num_planes", C.c_int, [_H]),
     ("lvc_plane_keys", C.c_int, [_H, C.c_void_p]),
     ("lvc_ensure_plane", C.c_int, [_H, C.c_uint16]),
@@ -543,6 +555,25 @@ class Handle:
         lik = np.zeros((self.G, 4), dtype=np.float64)
         self._check(self.lib.lvc_copy_dense(self.h, depth.ctypes.data, ad.ctypes.data, lik.ctypes.data))
         return depth, ad, lik
+
+    def consensus(self, min_depth: int, threshold: float, depths=(), p0: int = 0, p1: int = -1):
+        """lvc_consensus over [p0, p1) (p1 < 0: the whole contig): (consensus letters, statistics).  The statistics dict
+        holds the counters of lvc_consensus_stats and `depth_ge`, a list aligned with `depths`."""
+        if int(min_depth) < 0:
+            raise ValueError(f"min_depth must be >= 0, not {min_depth}")
+        thr = np.asarray(depths, dtype=np.int64).reshape(-1)
+        if thr.size and (thr.min() < 0 or thr.max() > 0xFFFFFFFF):
+            raise ValueError(f"depth thresholds must be in [0, 2^32): {list(depths)}")
+        thr = thr.astype(np.uint32)
+        n = self.G if p1 < 0 else max(int(p1) - int(p0), 0)
+        seq = np.zeros(max(n, 1), dtype=np.uint8)
+        st = ConsensusStats()
+        self._check(self.lib.lvc_consensus(self.h, int(p0), int(p1), int(min_depth), float(threshold),
+                                           thr.ctypes.data if thr.size else None, int(thr.size), seq.ctypes.data,
+                                           C.byref(st)))
+        out = {name: int(getattr(st, name)) for name in CONSENSUS_COUNTERS}
+        out["depth_ge"] = [int(st.depth_ge[i]) for i in range(min(thr.size, 8))]
+        return seq[:n].tobytes(), out
 
     # ---- tables
     def plane_keys(self) -> np.ndarray:

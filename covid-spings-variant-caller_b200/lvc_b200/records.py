@@ -100,3 +100,10 @@ def format_site_csv(depth: np.ndarray, ad: np.ndarray, ref: str) -> str:
             cells += [str(n), "%.4f" % (n / d)]
         rows.append(f"{p + 1},{ref[p]},{d}," + ",".join(cells))
     return "\n".join(rows) + "\n"
+
+
+def format_consensus_fasta(contig: str, consensus: str, width: int = 60) -> str:
+    """FASTA of a consensus (LiveVariantCaller.consensus): header `>contig`, the deletion calls '-' removed, `width`
+    letters per line."""
+    seq = consensus.replace("-", "")
+    return f">{contig}\n" + "".join(seq[i:i + width] + "\n" for i in range(0, len(seq), width))

@@ -164,6 +164,37 @@ class LiveVariantCaller:
         with open(path, "w") as fh:
             fh.write(records.format_site_csv(depth, ad, self._ref))
 
+    # ------------------------------------------------------------------ consensus + coverage (not in the reference API)
+    def consensus(self, minDepth: int = 10, threshold: float = 0.0) -> str:
+        """Consensus genome, one letter per reference position (include/lvc.h lvc_consensus): 'N' below minDepth, '-'
+        where deletions are the majority, IUPAC codes where the bases needed to reach `threshold` of the depth differ.
+        Computed on the device from the count tables; contains no insertions (they are not counted)."""
+        with self._lock:
+            seq, _ = self._handle.consensus(int(minDepth), float(threshold))
+        return seq.decode("ascii")
+
+    def write_consensus(self, outputFasta: str, minDepth: int = 10, threshold: float = 0.0):
+        """FASTA of `consensus()` with the deletion calls removed, 60 letters per line."""
+        with self._lock:
+            text = records.format_consensus_fasta(self._contig, self.consensus(minDepth, threshold))
+        with open(outputFasta, "w") as fh:
+            fh.write(text)
+
+    def coverage_summary(self, depths=(1, 10, 20, 100), minDepth: int = 10, threshold: float = 0.0) -> dict:
+        """Coverage and completeness of the contig: the counters of lvc_consensus_stats, `depth_ge` and `breadth`
+        ({depth: positions with at least that depth, as a count and as a fraction}), `mean_depth` and `completeness`
+        (the share of positions whose consensus letter is not 'N')."""
+        depths = [int(x) for x in depths]
+        with self._lock:
+            _, st = self._handle.consensus(int(minDepth), float(threshold), depths)
+        n = st["n_positions"]
+        out = {k: v for k, v in st.items() if k != "depth_ge"}
+        out["depth_ge"] = dict(zip(depths, st["depth_ge"]))
+        out["mean_depth"] = st["depth_sum"] / n
+        out["breadth"] = {x: c / n for x, c in zip(depths, st["depth_ge"])}
+        out["completeness"] = (n - st["n_N"]) / n
+        return out
+
     # ------------------------------------------------------------------ state <-> reference schema
     def _export_tables(self):
         h = self._handle

@@ -264,6 +264,37 @@ int lvc_set_genotype_range(lvc_handle* h, int64_t p0, int64_t p1);
 int lvc_copy_dense(lvc_handle* h, uint32_t* depth /*[G]*/, uint32_t* ad /*[G*4] A,C,G,T*/,
                    double* lik /*[G*4]*/);
 
+/* ---- consensus genome and coverage summary [EXT] ------------------------------------------------
+ * The reference gives neither; both are computed on the device from the count tables alone (no genotype pass, no
+ * first-seen ordinals), so the result is the same for any deposit kernel, batch form, checkpoint load or reduction.
+ * For each position p in [p0, p1):
+ *   nA, nC, nG, nT = sums over the group-0 planes of slots 0..3;  nO = sum over the group-1..3 planes and all four
+ *   slots (=, IUPAC letters, N read as bases);  nD = dels[p];  d = nA + nC + nG + nT + nO + nD (64-bit; the
+ *   totalDepth of `memory`, 0 where p is not in it).
+ *   d == 0 or d < min_depth                                         -> 'N'
+ *   members = (count, rank) for rank, count in enumerate(nA, nC, nG, nT, nD) if count > 0, sorted by count descending,
+ *             ties by rank (A < C < G < T < deletion); take members in that order until cum / d >= threshold (fp64
+ *             division); never reached (the rest of the depth is in other codes)   -> 'N'
+ *   deletion taken first                                            -> '-'
+ *   else "=ACMGRSVTWYHKDBN"[mask], mask = OR of (1 << rank) of the taken bases (A=1 C=2 G=4 T=8: the BAM nibble
+ *   alphabet is the IUPAC code of the mask; a deletion taken later is not in the mask).
+ * threshold 0 is a plain majority call; 0.5-0.75 gives mixed positions ambiguity codes.  Letters are uppercase.
+ * Insertions are not in the tables, so the consensus contains none.
+ * Statistics over the same range: n_positions, depth_sum, depth_max, n_low_depth (d < min_depth), n_N (every 'N'),
+ * n_deleted (every '-'), n_ambiguous (two- and three-base codes), n_mismatch (a single-base call other than the reference
+ * letter, where toupper(ref[p]) is A/C/G/T), depth_ge[i] (d >= depth_thresholds[i], i < n_thresholds; the rest 0).
+ * p1 < 0: the whole contig.  threshold outside [0, 1] or NaN, n_thresholds outside 0..8 or a range outside [0, G):
+ * LVC_EINVAL.  seq_out (p1 - p0 bytes) and stats_out may be NULL.  Synchronous: returns after the copy back.  The
+ * kernel runs on the handle's stream after everything enqueued before (lvc_push_batch_device_async included).
+ * After lvc_peer_attach or lvc_reduce_tables(LVC_REDUCE_SCATTER) a rank's tables hold its own slice only: call it with
+ * the range of lvc_position_slice. */
+typedef struct lvc_consensus_stats {
+    uint64_t n_positions, depth_sum, depth_max, n_low_depth, n_N, n_deleted, n_ambiguous, n_mismatch;
+    uint64_t depth_ge[8];
+} lvc_consensus_stats;                                                   /* 128 bytes */
+int lvc_consensus(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, double threshold,
+                  const uint32_t* depth_thresholds, int n_thresholds, uint8_t* seq_out, lvc_consensus_stats* stats_out);
+
 /* ---- table access: self.memory (live_variant_caller.py:31), checkpoints (:40-52), tests, NCCL ----
  * A "plane" holds, for one (allele group, quality) key, uint32 counts [G][4].  key = group<<8 | q;
  * group 0 = A,C,G,T (slots 0..3); groups 1..3 hold the other BAM nibble codes:
@@ -341,7 +372,7 @@ uint64_t lvc_launch_count(lvc_handle* h);
  * host admission dropped are never shipped */
 uint64_t lvc_h2d_payload_bytes(lvc_handle* h);
 /* per-kernel device time from CUDA events recorded on the handle's stream around every launch while
- * timing is on.  which: 0 = tiled deposit, 1 = general deposit, 2 = genotype.  Reading resets. */
+ * timing is on.  which: 0 = tiled deposit, 1 = general deposit, 2 = genotype, 3 = consensus.  Reading resets. */
 int lvc_set_timing(lvc_handle* h, int on);
 int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launches);
 int lvc_version(void);
