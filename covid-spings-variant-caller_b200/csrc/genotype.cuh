@@ -59,7 +59,7 @@ struct GenoParams {
     uint32_t cand_cap;
 };
 
-constexpr int kGenoThreads = 128;            // 32 positions x 4 allele slots (LPP = 1)
+constexpr int kGenoThreads = 128;            // 32 positions x 4 allele slots
 #ifndef LVC_GENO_BATCH
 #define LVC_GENO_BATCH 8
 #endif
@@ -101,11 +101,9 @@ struct PlaneConst {
     double le1, le2, le3, lo1, lo2, lo3, e;
 };
 
-// LPP lanes per (position, allele slot); the 4 slots of a position sit in 4 adjacent lanes and are combined with
-// shuffles.  With LPP > 1 (wide quality alphabets: ONT) lane `sub` of a slot takes the planes k = sub (mod LPP) and the
-// partial products are multiplied together by a shuffle tree first.  Alleles of the rare groups 1..3 are handled by
-// the same lanes in turn.
-template <int LPP, int NG>      // NG = 1: only the A/C/G/T group has planes (the usual case), 4: all groups
+// One lane per (position, allele slot); the 4 slots of a position sit in 4 adjacent lanes and are combined with
+// shuffles.  Alleles of the rare groups 1..3 are handled by the same lanes in turn.
+template <int NG>      // NG = 1: only the A/C/G/T group has planes (the usual case), 4: all groups
 __global__ void __launch_bounds__(kGenoThreads) k_genotype(GenoParams gp, const uint32_t* const* __restrict__ plane_ptrs,
                                                            const PlaneConst* __restrict__ pconst,
                                                            const uint32_t* __restrict__ dels,
@@ -117,7 +115,7 @@ __global__ void __launch_bounds__(kGenoThreads) k_genotype(GenoParams gp, const 
                                                            uint32_t* __restrict__ cand_count_next,
                                                            uint32_t* __restrict__ seen) {
     const int tid = threadIdx.x;
-    // per-plane constants in shared memory: every lane of a warp (LPP = 1) or every LPP-th lane reads the same entry
+    // per-plane constants in shared memory: every lane of a warp reads the same entry
     extern __shared__ __align__(16) unsigned char geno_smem[];
     PlaneConst* s_pc = reinterpret_cast<PlaneConst*>(geno_smem);
     // the per-plane constants were uploaded by a copy that precedes the previous kernel of the stream (or this launch,
@@ -133,15 +131,14 @@ __global__ void __launch_bounds__(kGenoThreads) k_genotype(GenoParams gp, const 
     asm volatile("griddepcontrol.launch_dependents;");        // the next deposit kernel may start reading its batch
     if (blockIdx.x == 0 && tid == 0) *cand_count_next = 0;
     const int slot = tid & 3;
-    const int sub = (tid >> 2) & (LPP - 1);
-    // the first position of a block is a multiple of 8 (a warp of the LPP = 1 variant writes one word of `seen`)
-    const int64_t p = (gp.p0 & ~7ll) + (int64_t)blockIdx.x * (kGenoThreads / (4 * LPP)) + (tid / (4 * LPP));
+    // the first position of a block is a multiple of 8 (a warp writes one word of `seen`)
+    const int64_t p = (gp.p0 & ~7ll) + (int64_t)blockIdx.x * (kGenoThreads / 4) + (tid / 4);
     const bool live = p >= gp.p0 && p < gp.p1;
     const int64_t pc = p < gp.p0 ? gp.p0 : (p < gp.p1 ? p : gp.p1 - 1);   // clamp: every lane takes part in the shuffles
     // requested now, used after the plane loop: deletion entries of the position and (for the hint) the first-seen cell
     const uint32_t dels_p = dels[pc];
     uint32_t first_p = kUnsetOrdinal;
-    if (LPP == 1 && seen && first[0]) first_p = first[0][pc * 4 + slot];
+    if (seen && first[0]) first_p = first[0][pc * 4 + slot];
     __syncthreads();
 
     AlleleStat st[NG];
@@ -153,15 +150,15 @@ __global__ void __launch_bounds__(kGenoThreads) k_genotype(GenoParams gp, const 
     for (int g = 0; g < NG; ++g) {
         // counts of up to kGenoBatch planes are requested together (one memory latency per batch, not per plane);
         // a count of 0 adds 0 to every sum, so nothing branches on the data
-        for (int k0 = gp.grp_begin[g] + sub; k0 < gp.grp_begin[g + 1]; k0 += kGenoBatch * LPP) {
+        for (int k0 = gp.grp_begin[g]; k0 < gp.grp_begin[g + 1]; k0 += kGenoBatch) {
             uint32_t cnt[kGenoBatch];
 #pragma unroll
             for (int j = 0; j < kGenoBatch; ++j)
-                cnt[j] = k0 + j * LPP < gp.grp_begin[g + 1] ? __ldcg(&plane_ptrs[k0 + j * LPP][pc * 4 + slot]) : 0u;
+                cnt[j] = k0 + j < gp.grp_begin[g + 1] ? __ldcg(&plane_ptrs[k0 + j][pc * 4 + slot]) : 0u;
 #pragma unroll
             for (int j = 0; j < kGenoBatch; ++j) {
-                if (k0 + j * LPP < gp.grp_begin[g + 1]) {                 // uniform over the lanes that share `sub`
-                    const PlaneConst& pcn = s_pc[k0 + j * LPP];
+                if (k0 + j < gp.grp_begin[g + 1]) {                       // uniform over the block
+                    const PlaneConst& pcn = s_pc[k0 + j];
                     const double nd = (double)cnt[j];
                     st[g].ad += cnt[j];
                     st[g].es = fma(nd, pcn.e, st[g].es);
@@ -172,16 +169,6 @@ __global__ void __launch_bounds__(kGenoThreads) k_genotype(GenoParams gp, const 
         }
         pe_dd[g] = acc3_fold(st[g].pe);
         p1_dd[g] = acc3_fold(st[g].p1);
-        if (LPP > 1 && gp.grp_begin[g + 1] > gp.grp_begin[g]) {
-            // partial sums of the LPP lanes of this (position, slot): lanes differ in bits 2.. of the lane index
-#pragma unroll
-            for (int d = 4; d < 4 * LPP; d <<= 1) {
-                pe_dd[g] = dd_add(pe_dd[g], dd_shfl_xor(pe_dd[g], d));
-                p1_dd[g] = dd_add(p1_dd[g], dd_shfl_xor(p1_dd[g], d));
-                st[g].es += __shfl_xor_sync(0xFFFFFFFFu, st[g].es, d);
-                st[g].ad += __shfl_xor_sync(0xFFFFFFFFu, st[g].ad, d);
-            }
-        }
     }
     // ---- combine the (up to 16) alleles of the position: log2 of the product of e over ALL of them
     constexpr bool has_other = NG > 1;
@@ -210,14 +197,14 @@ __global__ void __launch_bounds__(kGenoThreads) k_genotype(GenoParams gp, const 
     Ssum += __shfl_xor_sync(0xFFFFFFFFu, Ssum, 1);
     Ssum += __shfl_xor_sync(0xFFFFFFFFu, Ssum, 2);
     const double S = Ssum == 0.0 ? 1.0 : Ssum;                                   // live_variant_caller.py:146
-    if (LPP == 1 && seen) {
+    if (seen) {
         // hint for the deposit kernels (TableView::seen): which A/C/G/T alleles of these 8 positions have a first-seen
         // ordinal now -- no later batch can lower it.  Lane = position * 4 + slot is exactly the nibble layout.
         const bool has = live && first_p != kUnsetOrdinal;
         const uint32_t word = __ballot_sync(0xFFFFFFFFu, has);
         if ((tid & 31) == 0) seen[p >> 3] = word;
     }
-    if (!live || sub != 0) return;
+    if (!live) return;
     const uint32_t depth32 = (uint32_t)(depth > 0xFFFFFFFFull ? 0xFFFFFFFFull : depth);
     if (slot == 0) out_depth[p] = depth32;
     out_ad[p * 4 + slot] = st[0].ad;

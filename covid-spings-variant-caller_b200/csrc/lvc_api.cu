@@ -20,6 +20,7 @@
 #include "deposit_ont.cuh"
 #include "genotype.cuh"
 #include "consensus.cuh"
+#include "deposit_select.hpp"
 #include "overlap.hpp"
 #include "qcode.hpp"
 
@@ -52,9 +53,6 @@ struct lvc_handle {
     bool own_stream = false;
     std::string err;
     int impl = 0;
-    int geno_lpp_wide = 1;                   // lanes per (position, slot) of the genotype pass for wide quality alphabets on short contigs (LVC_GENO_LPP)
-    int long_impl = 6;                       // what impl 0 picks for long-read batches (LVC_LONG_IMPL = 3 or 6)
-    int tile_impl = 5;                       // what impl 0 (auto) picks for short-read batches (LVC_TILE_IMPL overrides)
     int sm_count = 148;
     uint64_t launches = 0;
     bool zero_copy_ok = true;                // read page-locked caller payload in place (LVC_ZERO_COPY=0 disables)
@@ -179,17 +177,56 @@ static TableView table_view(lvc_handle* h) {
     return tv;
 }
 
+// One kernel launch on the handle's stream, counted in lvc_launch_count.  `pdl`: programmatic stream serialization -- the
+// kernel may become resident while the previous kernel of the stream drains, so it must execute griddepcontrol.wait
+// before it reads or writes anything that kernel touches.
+static cudaError_t launch_kernel(lvc_handle* h, const void* kern, dim3 grid, dim3 block, size_t smem, bool pdl, void** args) {
+    cudaLaunchAttribute at;
+    at.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at.val.programmaticStreamSerializationAllowed = 1;
+    const cudaLaunchConfig_t cfg = {grid, block, smem, h->stream, &at, pdl ? 1u : 0u};
+    const cudaError_t e = cudaLaunchKernelExC(&cfg, kern, args);
+    if (e == cudaSuccess) h->launches++;
+    return e;
+}
+// the same with the arguments converted to the kernel's parameter types
+template <typename... P, typename... A>
+static cudaError_t launch_kernel(lvc_handle* h, void (*kern)(P...), dim3 grid, dim3 block, size_t smem, bool pdl, A&&... args) {
+    return [&](P... p) {
+        void* pargs[] = {&p...};
+        return launch_kernel(h, (const void*)kern, grid, block, smem, pdl, pargs);
+    }(std::forward<A>(args)...);
+}
+
+// Every instantiation of the tiled deposit kernels: by GE_ALL (threshold <= 0), and for generation 5 by PEER and by the
+// batch's payload form (phred bytes, quality codes, quality and base codes).  launch_deposit picks from these tables and
+// lvc_create raises the dynamic shared memory limit of every entry.
+using TileKernel = void (*)(BatchView, TableView, DepositParams, TileParams);
+static const TileKernel kTile3[2] = {k_deposit_tile<false>, k_deposit_tile<true>};
+static const TileKernel kTile4[2] = {k_deposit_tile4<false>, k_deposit_tile4<true>};
+static const TileKernel kTile5[2][2][3] = {
+    {{k_deposit_tile5<false, false>, k_deposit_tile5<false, false, true>, k_deposit_tile5<false, false, true, true>},
+     {k_deposit_tile5<false, true>, k_deposit_tile5<false, true, true>, k_deposit_tile5<false, true, true, true>}},
+    {{k_deposit_tile5<true, false>, k_deposit_tile5<true, false, true>, k_deposit_tile5<true, false, true, true>},
+     {k_deposit_tile5<true, true>, k_deposit_tile5<true, true, true>, k_deposit_tile5<true, true, true, true>}}};
+
+// allocate the first-seen table of allele group g if it has none yet (all cells unset); uploads its pointer
+static int ensure_first_table(lvc_handle* h, int g) {
+    if (h->d_first[g]) return LVC_OK;
+    const size_t bytes = ((size_t)h->G + kRowSlack) * 4 * sizeof(uint32_t);
+    CU(cudaMalloc(&h->d_first[g], bytes));
+    CU(cudaMemsetAsync(h->d_first[g], 0xFF, bytes, h->stream));
+    CU(cudaMemcpyAsync(h->d_first_arr + g, &h->d_first[g], sizeof(uint32_t*), cudaMemcpyHostToDevice, h->stream));
+    return LVC_OK;
+}
+
 // allocate a plane for `key` (and the group's first-seen table); uploads pointer + lut entry
 static int add_plane(lvc_handle* h, uint16_t key) {
     if (key >= kMaxKeys) return fail(h, LVC_EINVAL, "plane key %u out of range", key);
     if (h->lut[key] != kNoPlane) return LVC_OK;
-    const int g = key >> 8;
+    int rc = ensure_first_table(h, key >> 8);
+    if (rc) return rc;
     const size_t bytes = ((size_t)h->G + kRowSlack) * 4 * sizeof(uint32_t);
-    if (!h->d_first[g]) {
-        CU(cudaMalloc(&h->d_first[g], bytes));
-        CU(cudaMemsetAsync(h->d_first[g], 0xFF, bytes, h->stream));
-        CU(cudaMemcpyAsync(h->d_first_arr + g, &h->d_first[g], sizeof(uint32_t*), cudaMemcpyHostToDevice, h->stream));
-    }
     uint32_t* p = nullptr;
     CU(cudaMalloc(&p, bytes));
     CU(cudaMemsetAsync(p, 0, bytes, h->stream));
@@ -226,9 +263,6 @@ int lvc_create(lvc_handle** out, int device, int64_t ref_len, const uint8_t* ref
     for (int k = 0; k < kMaxKeys; ++k) h->lut[k] = kNoPlane;
     if (const char* zc = getenv("LVC_ZERO_COPY")) h->zero_copy_ok = atoi(zc) != 0;
     if (const char* zh = getenv("LVC_ZC_HEADERS")) h->zc_headers = atoi(zh) != 0;
-    if (const char* gl = getenv("LVC_GENO_LPP")) { const int v = atoi(gl); if (v == 1 || v == 2 || v == 4 || v == 8) h->geno_lpp_wide = v; }
-    if (const char* li = getenv("LVC_LONG_IMPL")) { const int v = atoi(li); if (v == 3 || v == 6) h->long_impl = v; }
-    if (const char* ti = getenv("LVC_TILE_IMPL")) { const int v = atoi(ti); if (v == 2 || v == 4 || v == 5) h->tile_impl = v; }
     auto body = [&]() -> int {
         CU(cudaSetDevice(device));
         cudaDeviceProp prop;
@@ -269,22 +303,10 @@ int lvc_create(lvc_handle** out, int device, int64_t ref_len, const uint8_t* ref
         CU(cudaMemsetAsync(h->d_out_lik, 0, G * 4 * sizeof(double), h->stream));
         CU(cudaMalloc(&h->d_cand_count, 2 * sizeof(uint32_t)));
         CU(cudaMemsetAsync(h->d_cand_count, 0, 2 * sizeof(uint32_t), h->stream));
-        CU(cudaFuncSetAttribute(k_deposit_tile<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile4<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile4SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile4<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile4SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<false, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<true, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
-        CU(cudaFuncSetAttribute(k_deposit_tile5<false, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
+        for (TileKernel k : kTile3) CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTileSmemBytes));
+        for (TileKernel k : kTile4) CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile4SmemBytes));
+        for (auto& by_peer : kTile5) for (auto& by_form : by_peer) for (TileKernel k : by_form)
+            CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTile5SmemBytes));
         CU(cudaStreamSynchronize(h->stream));
         return LVC_OK;
     };
@@ -424,109 +446,73 @@ static int launch_deposit(lvc_handle* h, const BatchView& bv, int replay, uint64
     dp.replay_keys = h->d_replay;
     const uint32_t n = bv.n_reads;
     if (n == 0) return LVC_OK;
-    // auto: batches of long reads (many CIGAR ops per read: ONT) take the warp-per-read kernel, short-read batches
-    // the tiled kernel
-    const bool long_reads = n_cigar_ops > 4ull * n;
-    // long reads: the CTA-cooperative kernel while the reads' ops fit its tables (<= 32 per read), else one warp per read
-    // (its cell indices are 32-bit: contigs below 2^30 columns)
-    const int long_impl = (n_cigar_ops <= 40ull * n && !replay && h->long_impl == 6 && h->G < (1ll << 30)) ? 6 : 3;
-    int impl = h->impl == 0 ? (long_reads ? long_impl : h->tile_impl) : h->impl;
-    if (h->peer_ranks > 1) {
-        // peer tables: only the generation-5 tiled kernel and the any-record kernels route their reductions
-        if (h->planes.size() != h->peer_planes_at_attach)
-            return fail(h, LVC_EINVAL, "a plane was added after lvc_peer_attach: export and attach again");
-        impl = (impl == 5 || (h->impl == 0 && !long_reads)) ? 5 : (long_reads ? 3 : 1);
-    }
-    // the tiled kernels' byte arithmetic assumes a primary quality and a threshold below 128
-    bool tile_ok = h->qprim < 128 && h->min_bq <= 128 && h->lut[h->qprim] != kNoPlane;
-    // quality-code batches (lvc_batch::qual_bits == 2): the generation-5 tiled kernel, or the any-record kernel
+    // quality-code batches: the code of the primary quality (4: none) and the other codes that pass the threshold
     const bool qc = bv.qbits == 2u;
     uint32_t qc_pcode = 4, qc_cold = 0;
-    if (qc) {
-        if (h->impl != 0 && h->impl != 1 && h->impl != 5)
-            return fail(h, LVC_EINVAL, "quality-code batches run on impl 0, 1 or 5 (selected: %d)", h->impl);
-        for (uint32_t c = 0; c < 4; ++c) {
-            const int v = (int)((bv.qdict >> (8 * c)) & 255u);
-            if (v == h->qprim && qc_pcode == 4) qc_pcode = c;
-        }
-        for (uint32_t c = 0; c < 4; ++c)
-            if (c != qc_pcode && (int)((bv.qdict >> (8 * c)) & 255u) >= h->min_bq) qc_cold |= 1u << c;
-        tile_ok = tile_ok && qc_pcode < 4;
-        impl = (impl == 1 || replay || !tile_ok) ? 1 : 5;
+    for (uint32_t c = 0; c < 4 && qc; ++c) {
+        const int v = (int)((bv.qdict >> (8 * c)) & 255u);
+        if (v == h->qprim && qc_pcode == 4) qc_pcode = c;
+        else if (v >= h->min_bq) qc_cold |= 1u << c;
     }
-    if (qc && impl == 1) {
-        { KernelTimer t(h, 1);
-          if (h->peer_ranks > 1) k_deposit_general<true><<<(n + 127) / 128, 128, 0, h->stream>>>(bv, tv, dp, n);
-          else k_deposit_general<false><<<(n + 127) / 128, 128, 0, h->stream>>>(bv, tv, dp, n); }
-        h->launches++;
-    } else if (impl == 6 && !replay && h->G < (1ll << 30)) {
+    DepositInputs in;
+    in.impl = h->impl; in.n_reads = n; in.n_cigar_ops = n_cigar_ops; in.replay = replay != 0; in.small_contig = h->G < (1ll << 30);
+    in.peer = h->peer_ranks > 1; in.planes_changed = h->planes.size() != h->peer_planes_at_attach;
+    // the tiled kernels' byte arithmetic assumes a primary quality and a threshold below 128
+    in.tile_ok = h->qprim < 128 && h->min_bq <= 128 && h->lut[h->qprim] != kNoPlane;
+    in.qc = qc; in.qc_prim_coded = qc_pcode < 4; in.base_codes = bv.sbits == 2u;
+    const DepositChoice choice = select_deposit(in);
+    if (choice.error == DepositError::planes_after_attach)
+        return fail(h, LVC_EINVAL, "a plane was added after lvc_peer_attach: export and attach again");
+    if (choice.error == DepositError::qc_impl)
+        return fail(h, LVC_EINVAL, "quality-code batches run on impl 0, 1 or 5 (selected: %d)", h->impl);
+    TileParams tp = make_tile_params(n, h->sm_count);
+    tp.qprim = (uint32_t)h->qprim; tp.prim_plane = h->lut[h->qprim]; tp.qc_pcode = qc_pcode & 3u; tp.qc_cold = qc_cold;
+    uint32_t rpc = 0;                           // k_deposit_ont: reads per CTA
+    void* last_arg = (void*)&n;                 // the tiled kernels take TileParams where the others take n
+    const bool peer = in.peer, ge_all = h->min_bq <= 0;
+    // programmatic stream serialization (pdl): the warp, ONT and generation-4/5 tiled kernels read their chunk headers or
+    // walk their CIGARs while the previous kernel of the stream drains, and wait for it before their first table access.
+    // The general and generation-3 kernels never wait: they start after the previous kernel has finished.
+    const void* kern = nullptr;
+    dim3 grid, block;
+    size_t smem = 0;
+    bool pdl = true;
+    int timer = 1;                              // KernelTimer slot: 0 tiled, 1 general / warp / ONT
+    switch (choice.kernel) {
+    case DepositKernel::general:
+        kern = (const void*)(peer ? k_deposit_general<true> : k_deposit_general<false>);
+        grid = dim3((n + 127) / 128); block = dim3(128); pdl = false;
+        break;
+    case DepositKernel::warp: {
+        const unsigned wpb = kWarpKernelThreads / 32;
+        kern = (const void*)(peer ? k_deposit_warp<true> : k_deposit_warp<false>);
+        grid = dim3((n + wpb - 1) / wpb); block = dim3(kWarpKernelThreads);
+        break;
+    }
+    case DepositKernel::ont: {
         // reads per CTA: as many as keep the CTA's unit list (16 query bases per unit) about three quarters full
         const uint64_t avg_q = std::max<uint64_t>(n_qual / n, 1);
-        const uint32_t rpc = (uint32_t)std::min<uint64_t>(kOntMaxReads, std::max<uint64_t>(1, (uint64_t)kOntMaxUnits * 12 / avg_q));
-        { KernelTimer t(h, 1);
-          cudaLaunchConfig_t cfg = {};
-          cfg.gridDim = dim3((n + rpc - 1) / rpc); cfg.blockDim = dim3(kOntThreads); cfg.stream = h->stream;
-          cudaLaunchAttribute at[1];
-          at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-          at[0].val.programmaticStreamSerializationAllowed = 1;
-          cfg.attrs = at; cfg.numAttrs = 1;
-          CU(cudaLaunchKernelEx(&cfg, k_deposit_ont, bv, tv, dp, n, rpc)); }
-        h->launches++;
-    } else if (impl == 3 || impl == 6 || ((replay || !tile_ok) && impl != 1 && long_reads)) {
-        { KernelTimer t(h, 1);
-          cudaLaunchConfig_t cfg = {};
-          const unsigned wpb = kWarpKernelThreads / 32;
-          cfg.gridDim = dim3((n + wpb - 1) / wpb); cfg.blockDim = dim3(kWarpKernelThreads); cfg.stream = h->stream;
-          cudaLaunchAttribute at[1];
-          at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-          at[0].val.programmaticStreamSerializationAllowed = 1;
-          cfg.attrs = at; cfg.numAttrs = 1;
-          if (h->peer_ranks > 1) CU(cudaLaunchKernelEx(&cfg, k_deposit_warp<true>, bv, tv, dp, n));
-          else CU(cudaLaunchKernelEx(&cfg, k_deposit_warp<false>, bv, tv, dp, n)); }
-        h->launches++;
-    } else if (impl == 1 || replay || !tile_ok) {
-        { KernelTimer t(h, 1);
-          if (h->peer_ranks > 1) k_deposit_general<true><<<(n + 127) / 128, 128, 0, h->stream>>>(bv, tv, dp, n);
-          else k_deposit_general<false><<<(n + 127) / 128, 128, 0, h->stream>>>(bv, tv, dp, n); }
-        h->launches++;
-    } else {
-        TileParams tp = make_tile_params(n, h->sm_count);
-        tp.qprim = (uint32_t)h->qprim;
-        tp.prim_plane = h->lut[h->qprim];
-        tp.qc_pcode = qc_pcode & 3u;
-        tp.qc_cold = qc_cold;
-        { KernelTimer t(h, 0);
-          if (impl == 4 || impl == 5) {
-              // programmatic stream serialization: the chunk headers are read (and dead chunks retire) while the
-              // previous kernel of the stream drains; the kernel waits for it before its first table access
-              cudaLaunchConfig_t cfg = {};
-              cfg.gridDim = dim3(impl == 5 ? (n + kT5Reads - 1) / kT5Reads : tp.grid);
-              cfg.blockDim = dim3(impl == 5 ? kT5Threads : kTileThreads);
-              cfg.dynamicSmemBytes = impl == 5 ? kTile5SmemBytes : kTile4SmemBytes;
-              cfg.stream = h->stream;
-              cudaLaunchAttribute at[1];
-              at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-              at[0].val.programmaticStreamSerializationAllowed = 1;
-              cfg.attrs = at; cfg.numAttrs = 1;
-              if (impl == 5) {
-                  using T5 = decltype(&k_deposit_tile5<false, false>);
-                  static const T5 t5[2][2][2] = {{{k_deposit_tile5<false, false>, k_deposit_tile5<false, false, true>},
-                                                  {k_deposit_tile5<false, true>, k_deposit_tile5<false, true, true>}},
-                                                 {{k_deposit_tile5<true, false>, k_deposit_tile5<true, false, true>},
-                                                  {k_deposit_tile5<true, true>, k_deposit_tile5<true, true, true>}}};
-                  static const T5 t5b2[2][2] = {{k_deposit_tile5<false, false, true, true>, k_deposit_tile5<false, true, true, true>},
-                                                {k_deposit_tile5<true, false, true, true>, k_deposit_tile5<true, true, true, true>}};
-                  if (qc && bv.sbits == 2u) CU(cudaLaunchKernelEx(&cfg, t5b2[h->min_bq <= 0 ? 1 : 0][h->peer_ranks > 1 ? 1 : 0], bv, tv, dp, tp));
-                  else
-                  CU(cudaLaunchKernelEx(&cfg, t5[h->min_bq <= 0 ? 1 : 0][h->peer_ranks > 1 ? 1 : 0][qc ? 1 : 0], bv, tv, dp, tp));
-              } else if (h->min_bq <= 0) CU(cudaLaunchKernelEx(&cfg, k_deposit_tile4<true>, bv, tv, dp, tp));
-              else CU(cudaLaunchKernelEx(&cfg, k_deposit_tile4<false>, bv, tv, dp, tp));
-          } else if (h->min_bq <= 0)
-              k_deposit_tile<true><<<tp.grid, kTileThreads, kTileSmemBytes, h->stream>>>(bv, tv, dp, tp);
-          else
-              k_deposit_tile<false><<<tp.grid, kTileThreads, kTileSmemBytes, h->stream>>>(bv, tv, dp, tp); }
-        h->launches++;
+        rpc = (uint32_t)std::min<uint64_t>(kOntMaxReads, std::max<uint64_t>(1, (uint64_t)kOntMaxUnits * 12 / avg_q));
+        kern = (const void*)k_deposit_ont;
+        grid = dim3((n + rpc - 1) / rpc); block = dim3(kOntThreads);
+        break;
     }
+    case DepositKernel::tile3:
+        kern = (const void*)kTile3[ge_all];
+        grid = dim3(tp.grid); block = dim3(kTileThreads); smem = kTileSmemBytes; pdl = false; timer = 0; last_arg = &tp;
+        break;
+    case DepositKernel::tile4:
+        kern = (const void*)kTile4[ge_all];
+        grid = dim3(tp.grid); block = dim3(kTileThreads); smem = kTile4SmemBytes; timer = 0; last_arg = &tp;
+        break;
+    case DepositKernel::tile5:
+        kern = (const void*)kTile5[ge_all][peer][choice.t5_form];
+        grid = dim3((n + kT5Reads - 1) / kT5Reads); block = dim3(kT5Threads); smem = kTile5SmemBytes; timer = 0; last_arg = &tp;
+        break;
+    }
+    void* args[] = {(void*)&bv, &tv, &dp, last_arg, &rpc};
+    { KernelTimer t(h, timer);
+      CU(launch_kernel(h, kern, grid, block, smem, pdl, args)); }
     CU(cudaGetLastError());
     return LVC_OK;
 }
@@ -541,19 +527,16 @@ static int deposit_with_replay(lvc_handle* h, const BatchView& bv, uint64_t n_ci
     CU(cudaMemcpyAsync(h->h_status, h->d_status, ST_WORDS * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
     CU(cudaMemcpyAsync(h->h_status + ST_WORDS, h->d_newkeys, 32 * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
     if (account) {
-        // zero-copy push: what crosses PCIe is what the kernel requests -- per chunk of 256 reads the 16-byte groups
-        // of the byte extent [first live read, end of last live read) (dead reads in between ride along; chunks with no
-        // live read request nothing).  Counted here, on the host, while the kernel runs.
+        // zero-copy push: what crosses PCIe is what the kernel requests -- per chunk of kT5Reads reads the 16-byte
+        // groups of the byte extent [first live read, end of last live read) (dead reads in between ride along; chunks
+        // with no live read request nothing).  Counted here, on the host, while the kernel runs.
         uint64_t moved = 0;
         const size_t n = account->n_reads;
-        const size_t chunk = h->tile_impl == 5 ? (size_t)kT5Reads : (size_t)kTileReads;
-        for (size_t c0 = 0; c0 < n; c0 += chunk) {
-            const size_t c1 = std::min(n, c0 + chunk);
+        for (size_t c0 = 0; c0 < n; c0 += kT5Reads) {
+            const size_t c1 = std::min(n, c0 + kT5Reads);
             uint64_t lo = ~0ull, hi = 0;
             for (size_t i = c0; i < c1; ++i) {
-                const uint32_t f = account->flag[i];
-                const bool live = (account->keep[i] & 1u) && !(f & kFlagFilter) && (int)account->mapq[i] >= h->min_mq &&
-                                  !((f & 1u) && !(f & 2u));
+                const bool live = read_passes_filter(account->flag[i], account->mapq[i], account->keep[i], h->min_mq);
                 if (live) { lo = std::min<uint64_t>(lo, account->seq_off[i]); hi = std::max<uint64_t>(hi, account->seq_off[i + 1]); }
             }
             if (hi > lo) { const uint64_t q = ((hi + 15) & ~15ull) - (lo & ~15ull); moved += (account->qual_bits == 2u ? q / 4 : q) + ((account->seq_form & 255u) == 2u ? q / 4 : q / 2); }
@@ -653,12 +636,17 @@ static int validate_batch(lvc_handle* h, const lvc_batch* b) {
     return LVC_OK;
 }
 
-// the batch's quality form as the kernels see it
-static void set_quality_form(BatchView& bv, const lvc_batch* b) {
+// the batch as the kernels see it: the caller's arrays and the batch's quality form
+static BatchView batch_view(const lvc_batch* b) {
+    BatchView bv;
+    bv.n_reads = b->n_reads;
+    bv.pos = b->pos; bv.flag = b->flag; bv.mapq = b->mapq; bv.keep = b->keep;
+    bv.cigar_off = b->cigar_off; bv.cigar = b->cigar; bv.seq_off = b->seq_off; bv.seq4 = b->seq4; bv.qual = b->qual;
     bv.qbits = b->qual_bits == 2u ? 2u : 0u;
     bv.sbits = (b->seq_form & 255u) == 2u ? 2u : 0u;
     bv.qdict = (uint32_t)b->qual_dict[0] | ((uint32_t)b->qual_dict[1] << 8) | ((uint32_t)b->qual_dict[2] << 16) |
                ((uint32_t)b->qual_dict[3] << 24);
+    return bv;
 }
 
 int lvc_push_batch(lvc_handle* h, const lvc_batch* b) {
@@ -766,8 +754,7 @@ int lvc_push_batch(lvc_handle* h, const lvc_batch* b) {
     }
     rc = premap_host(h, b);
     if (rc) return rc;
-    BatchView bv;
-    bv.n_reads = b->n_reads;
+    BatchView bv = batch_view(b);
     bv.pos = (const int32_t*)h->b_pos.p;       bv.flag = (const uint16_t*)h->b_flag.p;
     bv.mapq = (const uint8_t*)h->b_mapq.p;     bv.keep = (const uint8_t*)h->b_keep.p;
     bv.cigar_off = (const uint32_t*)h->b_coff.p; bv.cigar = (const uint32_t*)h->b_cig.p;
@@ -779,7 +766,6 @@ int lvc_push_batch(lvc_handle* h, const lvc_batch* b) {
         bv.hdr_lazy = 1;
     }
     bv.qual = dev_qual;
-    set_quality_form(bv, b);
     return deposit_with_replay(h, bv, b->n_cigar_ops, b->n_qual_bytes, zero_copy ? b : nullptr);
 }
 
@@ -789,11 +775,7 @@ int lvc_push_batch_device(lvc_handle* h, const lvc_batch* b) {
     if (rc) return rc;
     if (b->n_reads == 0) return LVC_OK;
     CU(cudaSetDevice(h->device));
-    BatchView bv;
-    bv.n_reads = b->n_reads;
-    bv.pos = b->pos; bv.flag = b->flag; bv.mapq = b->mapq; bv.keep = b->keep;
-    bv.cigar_off = b->cigar_off; bv.cigar = b->cigar; bv.seq_off = b->seq_off; bv.seq4 = b->seq4; bv.qual = b->qual;
-    set_quality_form(bv, b);
+    const BatchView bv = batch_view(b);
     rc = premap_device(h, b);
     if (rc) return rc;
     return deposit_with_replay(h, bv, b->n_cigar_ops, b->n_qual_bytes);
@@ -807,11 +789,7 @@ int lvc_push_batch_device_async(lvc_handle* h, const lvc_batch* b) {
     CU(cudaSetDevice(h->device));
     if ((uint64_t)h->ordinal + b->n_reads >= 0xFFFFFFFFull)
         return fail(h, LVC_ERANGE, "first-seen ordinal space (2^32-1 reads per handle) exhausted");
-    BatchView bv;
-    bv.n_reads = b->n_reads;
-    bv.pos = b->pos; bv.flag = b->flag; bv.mapq = b->mapq; bv.keep = b->keep;
-    bv.cigar_off = b->cigar_off; bv.cigar = b->cigar; bv.seq_off = b->seq_off; bv.seq4 = b->seq4; bv.qual = b->qual;
-    set_quality_form(bv, b);
+    const BatchView bv = batch_view(b);
     if (h->qprim == 255) {
         // the first push of this handle is an asynchronous one (peer tables: nothing may be deposited before the tables
         // are mapped): elect the tiled kernel's primary quality now (one small copy + stream synchronisation)
@@ -866,22 +844,29 @@ int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launc
 // ------------------------------------------------------------------------------------------------
 // genotype
 // ------------------------------------------------------------------------------------------------
-static int genotype_enqueue(lvc_handle* h, int64_t min_total_depth, int64_t min_allele_depth, double min_ratio,
-                            const double* e_lut, const double* om_lut, uint32_t flags) {
+// the planes ordered by key -- group 0 (A/C/G/T) first, then groups 1..3 -- with their keys; the planes of group g are
+// [grp_begin[g], grp_begin[g + 1])
+static void ordered_planes(const lvc_handle* h, std::vector<uint32_t*>& ptrs, std::vector<uint16_t>& keys, int grp_begin[5]) {
     const int np = (int)h->planes.size();
-    // order planes: group 0 first (register path), then the rest
     std::vector<int> order(np);
     for (int i = 0; i < np; ++i) order[i] = i;
     std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return h->plane_key[a] < h->plane_key[b]; });
-    std::vector<uint32_t*> ptrs(std::max(np, 1));
-    std::vector<uint16_t> keys(std::max(np, 1));
-    int grp_begin[5] = {0, 0, 0, 0, 0};
+    ptrs.assign(std::max(np, 1), nullptr);
+    keys.assign(std::max(np, 1), 0);
+    for (int g = 0; g < 5; ++g) grp_begin[g] = 0;
     for (int i = 0; i < np; ++i) {
         ptrs[i] = h->planes[order[i]];
         keys[i] = h->plane_key[order[i]];
         grp_begin[(keys[i] >> 8) + 1] = i + 1;
     }
     for (int g = 1; g <= 4; ++g) grp_begin[g] = std::max(grp_begin[g], grp_begin[g - 1]);
+}
+
+static int genotype_enqueue(lvc_handle* h, int64_t min_total_depth, int64_t min_allele_depth, double min_ratio,
+                            const double* e_lut, const double* om_lut, uint32_t flags) {
+    const int np = (int)h->planes.size();
+    std::vector<uint32_t*> ptrs; std::vector<uint16_t> keys; int grp_begin[5];
+    ordered_planes(h, ptrs, keys, grp_begin);
     int rc = ensure(h, h->g_order_ptrs, ptrs.size() * sizeof(uint32_t*));
     if (rc) return rc;
     rc = ensure(h, h->g_order_keys, keys.size() * sizeof(uint16_t));
@@ -935,15 +920,10 @@ static int genotype_enqueue(lvc_handle* h, int64_t min_total_depth, int64_t min_
     gp.G = h->G; gp.p0 = h->geno_p0; gp.p1 = h->geno_p1 < 0 ? h->G : h->geno_p1; gp.min_total_depth = min_total_depth; gp.min_allele_depth = min_allele_depth;
     gp.min_ratio = min_ratio; gp.flags = flags; gp.n_planes = np; gp.cand_cap = h->cand_cap;
     for (int g = 0; g < 5; ++g) gp.grp_begin[g] = grp_begin[g];
-    const int threads = kGenoThreads;
-    // wide quality alphabets (ONT: dozens of planes) on a short contig: LPP lanes share the planes of one (position,
-    // slot) so that the grid still fills the GPU (a SARS-CoV-2 contig is only 120 k (position, slot) threads)
-    // wide quality alphabets (ONT: dozens of planes) on a short contig: one lane per (position, slot) measured best on
-    // B200 (config 3, 61 planes: 19 us; 2 / 4 / 8 lanes sharing the planes of a slot: 23 / 27 / 36 us; the 4 warps of a
-    // block sharing 8 positions: 23 us) -- the pass is bound by its fixed latency chain, not by loads in flight
-    int lpp = 1;
-    if (grp_begin[1] - grp_begin[0] >= 16 && gp.p1 - gp.p0 <= (1 << 19)) lpp = h->geno_lpp_wide;
-    const int ppb = threads / (4 * lpp);                      // positions per block
+    // one lane per (position, slot), also for wide quality alphabets (ONT: dozens of planes) on a short contig: measured
+    // best on B200 (config 3, 61 planes: 19 us; 2 / 4 / 8 lanes sharing the planes of a slot: 23 / 27 / 36 us; the 4 warps
+    // of a block sharing 8 positions: 23 us) -- the pass is bound by its fixed latency chain, not by loads in flight
+    const int ppb = kGenoThreads / 4;                         // positions per block
     const unsigned blocks = (unsigned)((gp.p1 - (gp.p0 & ~7ll) + ppb - 1) / ppb);          // position 0 of a block is a multiple of 8
     if (gp.p1 <= gp.p0) { h->last_cand_count = 0; h->geno_pending = false; return LVC_OK; }
     {
@@ -953,29 +933,17 @@ static int genotype_enqueue(lvc_handle* h, int64_t min_total_depth, int64_t min_
         // candidate counter alternates between two words, each call clearing the other one.
         KernelTimer t(h, 2);
         h->cand_slot ^= 1;
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(blocks); cfg.blockDim = dim3(threads); cfg.dynamicSmemBytes = 0; cfg.stream = h->stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        const bool other_groups = grp_begin[4] > grp_begin[1];
-        using GenoKernel = decltype(&k_genotype<1, 1>);
-        static const GenoKernel kerns[4][2] = {{k_genotype<1, 1>, k_genotype<1, 4>}, {k_genotype<2, 1>, k_genotype<2, 4>},
-                                               {k_genotype<4, 1>, k_genotype<4, 4>}, {k_genotype<8, 1>, k_genotype<8, 4>}};
-        const GenoKernel kern = kerns[lpp == 8 ? 3 : (lpp == 4 ? 2 : (lpp == 2 ? 1 : 0))][other_groups ? 1 : 0];
-        cfg.dynamicSmemBytes = (size_t)np * sizeof(PlaneConst);
-        if (cfg.dynamicSmemBytes > 48 * 1024) {        // > 877 planes: never seen, allowed (1024 keys x 56 B = 57 KB)
+        const auto kern = grp_begin[4] > grp_begin[1] ? k_genotype<4> : k_genotype<1>;
+        const size_t smem = (size_t)np * sizeof(PlaneConst);
+        if (smem > 48 * 1024) {        // > 877 planes: never seen, allowed (1024 keys x 56 B = 57 KB)
             CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kMaxKeys * sizeof(PlaneConst))));
         }
-        CU(cudaLaunchKernelEx(&cfg, kern, gp, (const uint32_t* const*)h->g_order_ptrs.p,
-                              (const PlaneConst*)h->g_pconst.p, (const uint32_t*)h->d_dels, (const uint8_t*)h->d_ref,
-                              (const uint32_t* const*)h->d_first_arr, h->d_out_depth, h->d_out_ad, h->d_out_lik,
-                              (lvc_candidate*)h->g_cand.p, h->d_cand_count + h->cand_slot,
-                              h->d_cand_count + (h->cand_slot ^ 1),
-                              (lpp == 1 && h->d_seen && !h->seen_off) ? h->d_seen + 2 : (uint32_t*)nullptr));
+        CU(launch_kernel(h, kern, dim3(blocks), dim3(kGenoThreads), smem, true, gp, (const uint32_t* const*)h->g_order_ptrs.p,
+                         (const PlaneConst*)h->g_pconst.p, (const uint32_t*)h->d_dels, (const uint8_t*)h->d_ref,
+                         (const uint32_t* const*)h->d_first_arr, h->d_out_depth, h->d_out_ad, h->d_out_lik,
+                         (lvc_candidate*)h->g_cand.p, h->d_cand_count + h->cand_slot, h->d_cand_count + (h->cand_slot ^ 1),
+                         (h->d_seen && !h->seen_off) ? h->d_seen + 2 : (uint32_t*)nullptr));
     }
-    h->launches++;
     CU(cudaGetLastError());
     h->geno_pending = true;
     return LVC_OK;
@@ -1075,17 +1043,9 @@ int lvc_consensus(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, dou
     CU(cudaSetDevice(h->device));
     const int np = (int)h->planes.size();
     if (h->cons_planes_uploaded != (size_t)np) {     // planes are only ever appended: the count identifies the set
-        // order planes: group 0 first, then groups 1..3 (the genotype pass keeps its own list)
-        std::vector<int> order(np);
-        for (int i = 0; i < np; ++i) order[i] = i;
-        std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return h->plane_key[a] < h->plane_key[b]; });
-        std::vector<uint32_t*> ptrs(std::max(np, 1));
-        int grp_begin[5] = {0, 0, 0, 0, 0};
-        for (int i = 0; i < np; ++i) {
-            ptrs[i] = h->planes[order[i]];
-            grp_begin[(h->plane_key[order[i]] >> 8) + 1] = i + 1;
-        }
-        for (int g = 1; g <= 4; ++g) grp_begin[g] = std::max(grp_begin[g], grp_begin[g - 1]);
+        // the genotype pass keeps its own device copy of this list
+        std::vector<uint32_t*> ptrs; std::vector<uint16_t> keys; int grp_begin[5];
+        ordered_planes(h, ptrs, keys, grp_begin);
         int rc = ensure(h, h->c_order_ptrs, ptrs.size() * sizeof(uint32_t*));
         if (rc) return rc;
         CU(cudaMemcpyAsync(h->c_order_ptrs.p, ptrs.data(), ptrs.size() * sizeof(uint32_t*), cudaMemcpyHostToDevice, h->stream));
@@ -1110,9 +1070,8 @@ int lvc_consensus(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, dou
         const unsigned blocks = (unsigned)std::min<int64_t>((n + kConsThreads - 1) / kConsThreads, (int64_t)h->sm_count * 16);
         // launched without programmatic serialization: it starts after every earlier kernel of the stream has finished
         KernelTimer t(h, 3);
-        k_consensus<<<blocks, kConsThreads, 0, h->stream>>>(cp, (const uint32_t* const*)h->c_order_ptrs.p, h->d_dels, h->d_ref,
-                                                             (uint8_t*)h->c_seq.p, (unsigned long long*)h->c_stats.p);
-        h->launches++;
+        CU(launch_kernel(h, k_consensus, dim3(blocks), dim3(kConsThreads), 0, false, cp, (const uint32_t* const*)h->c_order_ptrs.p,
+                         h->d_dels, h->d_ref, (uint8_t*)h->c_seq.p, (unsigned long long*)h->c_stats.p));
         CU(cudaGetLastError());
     }
     if (seq_out && n > 0) CU(cudaMemcpyAsync(seq_out, h->c_seq.p, (size_t)n, cudaMemcpyDeviceToHost, h->stream));
@@ -1163,8 +1122,7 @@ static int import_u32(lvc_handle* h, uint32_t* d_dst, const uint32_t* src, size_
         uint32_t* tmp = nullptr;
         CU(cudaMalloc(&tmp, n * 4));
         CU(cudaMemcpyAsync(tmp, src, n * 4, cudaMemcpyHostToDevice, h->stream));
-        k_accumulate_u32<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(d_dst, tmp, n);
-        h->launches++;
+        CU(launch_kernel(h, k_accumulate_u32, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, false, d_dst, tmp, n));
         CU(cudaStreamSynchronize(h->stream));
         CU(cudaFree(tmp));
     }
@@ -1222,12 +1180,8 @@ int lvc_copy_first(lvc_handle* h, int group, uint32_t* dst) {
 int lvc_import_first(lvc_handle* h, int group, const uint32_t* src) {
     if (!h || !src || group < 0 || group > 3) return LVC_EINVAL;
     CU(cudaSetDevice(h->device));
-    if (!h->d_first[group]) {
-        const size_t bytes = ((size_t)h->G + kRowSlack) * 16;
-        CU(cudaMalloc(&h->d_first[group], bytes));
-        CU(cudaMemsetAsync(h->d_first[group], 0xFF, bytes, h->stream));
-        CU(cudaMemcpyAsync(h->d_first_arr + group, &h->d_first[group], sizeof(uint32_t*), cudaMemcpyHostToDevice, h->stream));
-    }
+    int rc = ensure_first_table(h, group);
+    if (rc) return rc;
     CU(cudaMemsetAsync(h->d_seen, 0, h->seen_words * sizeof(uint32_t), h->stream));      // the hint describes the old table
     CU(cudaMemcpyAsync(h->d_first[group], src, (size_t)h->G * 16, cudaMemcpyHostToDevice, h->stream));
     CU(cudaStreamSynchronize(h->stream));

@@ -125,7 +125,7 @@ __device__ __forceinline__ uint32_t* first_row(const TableView& tv, uint32_t gro
     return tv.first[group] + col * 4;
 }
 
-__device__ __forceinline__ bool read_passes_filter(uint32_t flag, uint32_t mapq, uint32_t keep, int min_mq) {
+__host__ __device__ __forceinline__ bool read_passes_filter(uint32_t flag, uint32_t mapq, uint32_t keep, int min_mq) {
     // pysam stepper "samtools": flag filter, mapq, ignore_orphans (SURVEY B2) + host admission bit
     if (!(keep & 1u)) return false;
     if (flag & kFlagFilter) return false;

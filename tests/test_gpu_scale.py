@@ -118,7 +118,8 @@ def test_live_batches_ont(lib):
 
 def test_config3_sized_ont_batches(lib):
     """SURVEY 8d config 3 at full batch size (74,758 reads, ~21 CIGAR ops each, qualities 2..90): two live batches
-    through the warp-per-read kernel and the 8-lane genotype pass, against the C oracle"""
+    through the automatic long-read deposit choice and the genotype pass over their wide quality alphabet, against the
+    C oracle"""
     from lvc_b200 import synth
     ref = synth.random_reference(29903, 20260199)
     batches = [synth.ont_batch_fast(20260200 + k, ref) for k in range(2)]
