@@ -20,6 +20,7 @@
 #include "deposit_ont.cuh"
 #include "genotype.cuh"
 #include "consensus.cuh"
+#include "insertions.cuh"
 #include "deposit_select.hpp"
 #include "overlap.hpp"
 #include "qcode.hpp"
@@ -113,9 +114,16 @@ struct lvc_handle {
     size_t cons_planes_uploaded = (size_t)-1;
     int cons_grp_begin[5] = {0, 0, 0, 0, 0};
 
+    // insertion counts (lvc_enable_insertions): ins.keys == nullptr while counting is off
+    InsTable ins = {nullptr, nullptr, nullptr, 0};
+    bool tables_touched = false;             // a push, import or reduction since lvc_create / lvc_reset
+    bool ins_uncovered = false;              // an import or reduction since lvc_reset: counts the insertion table lacks
+    DevBuf i_list, i_scratch;
+
     // optional per-kernel timing (CUDA events on the launching stream)
     bool timing = false;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[4];   // 0 tiled deposit, 1 general deposit, 2 genotype, 3 consensus
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[5];   // 0 tiled deposit, 1 general deposit, 2 genotype, 3 consensus,
+                                                              // 4 insertion counts
     std::vector<cudaEvent_t> ev_pool;
 };
 
@@ -332,13 +340,14 @@ void lvc_destroy(lvc_handle* h) {
     cudaFree(h->d_first_arr); cudaFree(h->d_newkeys); cudaFree(h->d_replay); cudaFree(h->d_status); cudaFree(h->d_keymap);
     if (h->h_status) cudaFreeHost(h->h_status);
     if (h->h_sample) cudaFreeHost(h->h_sample);
-    for (int w = 0; w < 4; ++w) for (auto& pr : h->ev[w]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
+    for (int w = 0; w < 5; ++w) for (auto& pr : h->ev[w]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
     for (auto e : h->ev_pool) cudaEventDestroy(e);
     cudaFree(h->d_elut); cudaFree(h->d_out_depth); cudaFree(h->d_out_ad); cudaFree(h->d_out_lik);
     cudaFree(h->d_cand_count);
+    cudaFree(h->ins.keys); cudaFree(h->ins.counts); cudaFree(h->ins.dropped);
     for (DevBuf* b : {&h->b_pos, &h->b_flag, &h->b_mapq, &h->b_keep, &h->b_coff, &h->b_cig, &h->b_soff, &h->b_seq,
                       &h->b_qual, &h->g_order_ptrs, &h->g_order_keys, &h->g_cand, &h->g_pconst, &h->c_order_ptrs,
-                      &h->c_seq, &h->c_stats})
+                      &h->c_seq, &h->c_stats, &h->i_list, &h->i_scratch})
         cudaFree(b->p);
     if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -380,6 +389,14 @@ int lvc_reset(lvc_handle* h) {
     CU(cudaMemsetAsync(h->d_out_depth, 0, G * sizeof(uint32_t), h->stream));
     CU(cudaMemsetAsync(h->d_out_ad, 0, G * 4 * sizeof(uint32_t), h->stream));
     CU(cudaMemsetAsync(h->d_out_lik, 0, G * 4 * sizeof(double), h->stream));
+    if (h->ins.keys) {
+        const size_t slots = (size_t)h->ins.mask + 1;
+        CU(cudaMemsetAsync(h->ins.keys, 0, slots * sizeof(ulonglong2), h->stream));
+        CU(cudaMemsetAsync(h->ins.counts, 0, slots * sizeof(uint32_t), h->stream));
+        CU(cudaMemsetAsync(h->ins.dropped, 0, sizeof(uint32_t), h->stream));
+    }
+    h->tables_touched = false;
+    h->ins_uncovered = false;
     h->ordinal = 0;
     CU(cudaStreamSynchronize(h->stream));
     return LVC_OK;
@@ -517,12 +534,28 @@ static int launch_deposit(lvc_handle* h, const BatchView& bv, int replay, uint64
     return LVC_OK;
 }
 
+// The insertion counts of one batch (lvc_enable_insertions), launched right behind its first deposit pass while the batch
+// buffers are valid.  Programmatic serialization lets it overlap the deposit's tail; it reads no table the deposit writes.
+static int launch_count_insertions(lvc_handle* h, const BatchView& bv) {
+    if (!h->ins.keys || bv.n_reads == 0) return LVC_OK;
+    InsCountParams cp;
+    cp.G = h->G; cp.min_bq = h->min_bq; cp.min_mq = h->min_mq;
+    { KernelTimer t(h, 4);
+      CU(launch_kernel(h, k_count_insertions, dim3((bv.n_reads + kInsThreads - 1) / kInsThreads), dim3(kInsThreads), 0, true,
+                       bv, h->ins, cp, bv.n_reads)); }
+    CU(cudaGetLastError());
+    return LVC_OK;
+}
+
 static int deposit_with_replay(lvc_handle* h, const BatchView& bv, uint64_t n_cigar_ops, uint64_t n_qual,
                                const lvc_batch* account = nullptr) {
     if ((uint64_t)h->ordinal + bv.n_reads >= 0xFFFFFFFFull)
         return fail(h, LVC_ERANGE, "first-seen ordinal space (2^32-1 reads per handle) exhausted");
+    h->tables_touched = true;
     CU(cudaMemsetAsync(h->d_status, 0, ST_WORDS * sizeof(uint32_t), h->stream));
     int rc = launch_deposit(h, bv, 0, n_cigar_ops, n_qual);
+    if (rc) return rc;
+    rc = launch_count_insertions(h, bv);           // once per batch: the replay pass below does not count again
     if (rc) return rc;
     CU(cudaMemcpyAsync(h->h_status, h->d_status, ST_WORDS * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
     CU(cudaMemcpyAsync(h->h_status + ST_WORDS, h->d_newkeys, 32 * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
@@ -796,7 +829,10 @@ int lvc_push_batch_device_async(lvc_handle* h, const lvc_batch* b) {
         rc = premap_device(h, b);
         if (rc) return rc;
     }
+    h->tables_touched = true;
     rc = launch_deposit(h, bv, 0, b->n_cigar_ops, b->n_qual_bytes);
+    if (rc) return rc;
+    rc = launch_count_insertions(h, bv);
     if (rc) return rc;
     h->ordinal += b->n_reads;
     return LVC_OK;
@@ -824,7 +860,8 @@ int lvc_set_timing(lvc_handle* h, int on) {
 }
 
 int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launches) {
-    if (!h || which < 0 || which > 3 || !ms_total || !n_launches) return LVC_EINVAL;
+    if (!h || which < 0 || which > 4 || !ms_total || !n_launches) return LVC_EINVAL;
+    if (which == 4 && !h->ins.keys) return fail(h, LVC_EINVAL, "timer 4 (insertion counts) needs lvc_enable_insertions");
     CU(cudaSetDevice(h->device));
     CU(cudaStreamSynchronize(h->stream));
     double tot = 0.0;
@@ -1028,6 +1065,21 @@ int lvc_copy_dense(lvc_handle* h, uint32_t* depth, uint32_t* ad, double* lik) {
 // ------------------------------------------------------------------------------------------------
 // consensus + coverage statistics
 // ------------------------------------------------------------------------------------------------
+// the ordered plane list of the consensus and insertion-call passes (the genotype pass keeps its own device copy)
+static int upload_consensus_planes(lvc_handle* h) {
+    const int np = (int)h->planes.size();
+    if (h->cons_planes_uploaded == (size_t)np) return LVC_OK;     // planes are only ever appended: the count identifies the set
+    std::vector<uint32_t*> ptrs; std::vector<uint16_t> keys; int grp_begin[5];
+    ordered_planes(h, ptrs, keys, grp_begin);
+    int rc = ensure(h, h->c_order_ptrs, ptrs.size() * sizeof(uint32_t*));
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(h->c_order_ptrs.p, ptrs.data(), ptrs.size() * sizeof(uint32_t*), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaStreamSynchronize(h->stream));             // `ptrs` goes out of scope
+    memcpy(h->cons_grp_begin, grp_begin, sizeof grp_begin);
+    h->cons_planes_uploaded = (size_t)np;
+    return LVC_OK;
+}
+
 int lvc_consensus(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, double threshold,
                   const uint32_t* depth_thresholds, int n_thresholds, uint8_t* seq_out, lvc_consensus_stats* stats_out) {
     NvtxRange nvtx_range("lvc_consensus");
@@ -1041,20 +1093,10 @@ int lvc_consensus(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, dou
         return fail(h, LVC_EINVAL, "consensus range [%lld, %lld) outside [0, %lld)", (long long)p0, (long long)p1,
                     (long long)h->G);
     CU(cudaSetDevice(h->device));
-    const int np = (int)h->planes.size();
-    if (h->cons_planes_uploaded != (size_t)np) {     // planes are only ever appended: the count identifies the set
-        // the genotype pass keeps its own device copy of this list
-        std::vector<uint32_t*> ptrs; std::vector<uint16_t> keys; int grp_begin[5];
-        ordered_planes(h, ptrs, keys, grp_begin);
-        int rc = ensure(h, h->c_order_ptrs, ptrs.size() * sizeof(uint32_t*));
-        if (rc) return rc;
-        CU(cudaMemcpyAsync(h->c_order_ptrs.p, ptrs.data(), ptrs.size() * sizeof(uint32_t*), cudaMemcpyHostToDevice, h->stream));
-        CU(cudaStreamSynchronize(h->stream));             // `ptrs` goes out of scope
-        memcpy(h->cons_grp_begin, grp_begin, sizeof grp_begin);
-        h->cons_planes_uploaded = (size_t)np;
-    }
+    int rc = upload_consensus_planes(h);
+    if (rc) return rc;
     const int64_t n = p1 - p0;
-    int rc = ensure(h, h->c_seq, (size_t)std::max<int64_t>(n, 1));
+    rc = ensure(h, h->c_seq, (size_t)std::max<int64_t>(n, 1));
     if (rc) return rc;
     rc = ensure(h, h->c_stats, CS_WORDS * sizeof(uint64_t));
     if (rc) return rc;
@@ -1088,6 +1130,136 @@ int lvc_consensus(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, dou
         *stats_out = s;
     }
     return LVC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// insertions in the consensus
+// ------------------------------------------------------------------------------------------------
+static_assert(sizeof(lvc_insertion) == sizeof(InsEntry) && sizeof(lvc_insertion) == 24, "lvc_insertion layout");
+
+int lvc_enable_insertions(lvc_handle* h, uint32_t max_keys) {
+    if (!h) return LVC_EINVAL;
+    if (max_keys == 0 || max_keys > (1u << 30))
+        return fail(h, LVC_EINVAL, "lvc_enable_insertions: max_keys %u outside 1..2^30", max_keys);
+    if (h->G > 0x7FFFFFFF) return fail(h, LVC_EINVAL, "lvc_enable_insertions: contig longer than 2^31 - 1");
+    if (h->peer_ranks > 1) return fail(h, LVC_EINVAL, "lvc_enable_insertions: refused on a handle with peer tables attached");
+    if (h->tables_touched)
+        return fail(h, LVC_EINVAL, "lvc_enable_insertions: the tables already hold counts; call it after lvc_create or lvc_reset");
+    CU(cudaSetDevice(h->device));
+    size_t slots = 1;
+    while (slots < 2 * (size_t)max_keys) slots <<= 1;
+    CU(cudaStreamSynchronize(h->stream));
+    cudaFree(h->ins.keys); cudaFree(h->ins.counts); cudaFree(h->ins.dropped);
+    h->ins = InsTable{nullptr, nullptr, nullptr, 0};
+    InsTable t = {nullptr, nullptr, nullptr, (uint32_t)(slots - 1)};
+    if (cudaMalloc(&t.keys, slots * sizeof(ulonglong2)) != cudaSuccess || cudaMalloc(&t.counts, slots * sizeof(uint32_t)) != cudaSuccess ||
+        cudaMalloc(&t.dropped, sizeof(uint32_t)) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(t.keys); cudaFree(t.counts);
+        return fail(h, LVC_ENOMEM, "lvc_enable_insertions: no device memory for %zu slots", slots);
+    }
+    h->ins = t;
+    CU(cudaMemsetAsync(t.keys, 0, slots * sizeof(ulonglong2), h->stream));
+    CU(cudaMemsetAsync(t.counts, 0, slots * sizeof(uint32_t), h->stream));
+    CU(cudaMemsetAsync(t.dropped, 0, sizeof(uint32_t), h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    return LVC_OK;
+}
+
+// the conditions both queries share: counting on, tables covered by the counts, nothing dropped
+static int insertions_queryable(lvc_handle* h) {
+    if (!h->ins.keys) return fail(h, LVC_EINVAL, "insertion counting is off (lvc_enable_insertions)");
+    if (h->ins_uncovered)
+        return fail(h, LVC_EINVAL, "the tables hold imported or reduced counts that the insertion counts do not cover; "
+                    "lvc_reset starts over");
+    CU(cudaMemcpyAsync(h->h_status, h->ins.dropped, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    const uint32_t dropped = h->h_status[0];
+    if (dropped)
+        return fail(h, LVC_ENOMEM, "%u insertion(s) found no free slot in the insertion table (%u slots); enable counting with "
+                    "a larger max_keys", dropped, h->ins.mask + 1);
+    return LVC_OK;
+}
+
+static bool insertion_before(const lvc_insertion& a, const lvc_insertion& b) {
+    if (a.pos != b.pos) return a.pos < b.pos;
+    if (a.len != b.len) return a.len < b.len;
+    return a.seq < b.seq;
+}
+
+// n entries of the device list -> sorted, the first min(n, cap) into out
+static int copy_sorted(lvc_handle* h, uint32_t n, lvc_insertion* out, uint32_t cap) {
+    std::vector<lvc_insertion> v(n);
+    if (n) CU(cudaMemcpyAsync(v.data(), h->i_list.p, (size_t)n * sizeof(lvc_insertion), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    std::sort(v.begin(), v.end(), insertion_before);
+    if (out) std::copy(v.begin(), v.begin() + std::min(n, cap), out);
+    return LVC_OK;
+}
+
+int lvc_copy_insertions(lvc_handle* h, lvc_insertion* out, uint32_t cap, uint32_t* n_out) {
+    NvtxRange nvtx_range("lvc_copy_insertions");
+    if (!h || !n_out || (cap && !out)) return LVC_EINVAL;
+    CU(cudaSetDevice(h->device));
+    int rc = insertions_queryable(h);
+    if (rc) return rc;
+    const size_t slots = (size_t)h->ins.mask + 1;
+    rc = ensure(h, h->i_list, slots * sizeof(lvc_insertion) + sizeof(uint32_t));
+    if (rc) return rc;
+    uint32_t* d_n = (uint32_t*)((uint8_t*)h->i_list.p + slots * sizeof(lvc_insertion));
+    CU(cudaMemsetAsync(d_n, 0, sizeof(uint32_t), h->stream));
+    CU(launch_kernel(h, k_insertion_list, dim3((unsigned)((slots + kInsScanThreads - 1) / kInsScanThreads)), dim3(kInsScanThreads),
+                     0, false, h->ins, (InsEntry*)h->i_list.p, (uint32_t)slots, d_n));
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(h->h_status, d_n, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    *n_out = h->h_status[0];
+    return copy_sorted(h, *n_out, out, cap);
+}
+
+int lvc_insertion_calls(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, double threshold, lvc_insertion* out,
+                        uint32_t cap, uint32_t* n_out) {
+    NvtxRange nvtx_range("lvc_insertion_calls");
+    if (!h || !n_out || (cap && !out)) return LVC_EINVAL;
+    if (!(threshold >= 0.0 && threshold <= 1.0))
+        return fail(h, LVC_EINVAL, "insertion calls: threshold %g outside [0, 1]", threshold);
+    if (p1 < 0) { p0 = 0; p1 = h->G; }
+    if (p0 < 0 || p1 > h->G || p0 > p1)
+        return fail(h, LVC_EINVAL, "insertion calls: range [%lld, %lld) outside [0, %lld)", (long long)p0, (long long)p1,
+                    (long long)h->G);
+    CU(cudaSetDevice(h->device));
+    int rc = insertions_queryable(h);
+    if (rc) return rc;
+    rc = upload_consensus_planes(h);
+    if (rc) return rc;
+    const size_t slots = (size_t)h->ins.mask + 1;
+    const size_t n = (size_t)(p1 - p0);
+    // per-position scratch: total, unresolved, best, number of keys at the best
+    rc = ensure(h, h->i_scratch, std::max<size_t>(n, 1) * 4 * sizeof(uint32_t));
+    if (rc) return rc;
+    rc = ensure(h, h->i_list, slots * sizeof(lvc_insertion) + sizeof(uint32_t));
+    if (rc) return rc;
+    uint32_t* sc = (uint32_t*)h->i_scratch.p;
+    uint32_t* d_n = (uint32_t*)((uint8_t*)h->i_list.p + slots * sizeof(lvc_insertion));
+    CU(cudaMemsetAsync(sc, 0, std::max<size_t>(n, 1) * 4 * sizeof(uint32_t), h->stream));
+    CU(cudaMemsetAsync(d_n, 0, sizeof(uint32_t), h->stream));
+    if (n > 0) {
+        const dim3 grid((unsigned)((slots + kInsScanThreads - 1) / kInsScanThreads)), block(kInsScanThreads);
+        uint32_t *total = sc, *unres = sc + n, *best = sc + 2 * n, *n_best = sc + 3 * n;
+        InsCallParams ip;
+        ip.p0 = p0; ip.p1 = p1; ip.min_depth = min_depth; ip.threshold = threshold;
+        for (int g = 0; g < 5; ++g) ip.grp_begin[g] = h->cons_grp_begin[g];
+        CU(launch_kernel(h, k_insertion_tally, grid, block, 0, false, h->ins, p0, p1, total, unres, best));
+        CU(launch_kernel(h, k_insertion_ties, grid, block, 0, false, h->ins, p0, p1, (const uint32_t*)best, n_best));
+        CU(launch_kernel(h, k_insertion_call, grid, block, 0, false, h->ins, ip, (const uint32_t* const*)h->c_order_ptrs.p,
+                         (const uint32_t*)h->d_dels, (const uint32_t*)total, (const uint32_t*)unres, (const uint32_t*)best,
+                         (const uint32_t*)n_best, (InsEntry*)h->i_list.p, d_n));
+        CU(cudaGetLastError());
+    }
+    CU(cudaMemcpyAsync(h->h_status, d_n, sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    *n_out = h->h_status[0];
+    return copy_sorted(h, *n_out, out, cap);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1140,6 +1312,7 @@ int lvc_copy_plane(lvc_handle* h, uint16_t key, uint32_t* dst) {
 
 int lvc_import_plane(lvc_handle* h, uint16_t key, const uint32_t* src, int accumulate) {
     if (!h || !src) return LVC_EINVAL;
+    h->tables_touched = h->ins_uncovered = true;
     CU(cudaSetDevice(h->device));
     int rc = add_plane(h, key);
     if (rc) return rc;
@@ -1155,6 +1328,7 @@ int lvc_copy_dels(lvc_handle* h, uint32_t* dst) {
 }
 int lvc_import_dels(lvc_handle* h, const uint32_t* src, int accumulate) {
     if (!h || !src) return LVC_EINVAL;
+    h->tables_touched = h->ins_uncovered = true;
     CU(cudaSetDevice(h->device));
     return import_u32(h, h->d_dels, src, (size_t)h->G, accumulate);
 }
@@ -1167,6 +1341,7 @@ int lvc_copy_covdiff(lvc_handle* h, int32_t* dst) {
 }
 int lvc_import_covdiff(lvc_handle* h, const int32_t* src, int accumulate) {
     if (!h || !src) return LVC_EINVAL;
+    h->tables_touched = h->ins_uncovered = true;
     CU(cudaSetDevice(h->device));
     return import_u32(h, (uint32_t*)h->d_covdiff, (const uint32_t*)src, (size_t)h->G + 1, accumulate);
 }
@@ -1179,6 +1354,7 @@ int lvc_copy_first(lvc_handle* h, int group, uint32_t* dst) {
 }
 int lvc_import_first(lvc_handle* h, int group, const uint32_t* src) {
     if (!h || !src || group < 0 || group > 3) return LVC_EINVAL;
+    h->tables_touched = h->ins_uncovered = true;
     CU(cudaSetDevice(h->device));
     int rc = ensure_first_table(h, group);
     if (rc) return rc;

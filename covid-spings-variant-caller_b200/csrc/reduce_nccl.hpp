@@ -110,6 +110,7 @@ int lvc_reduce_tables(lvc_handle* h, void* nccl_comm, int n_ranks, int rank, int
     CU(cudaSetDevice(h->device));
     h->last_exchange_bytes = 0;
     if (n_ranks == 1) return LVC_OK;
+    h->tables_touched = h->ins_uncovered = true;      // the other ranks' counts arrive without their insertions
     // ---- (1) agree on the set of (allele group, quality) planes: byte-wise MAX of the 1024-key presence map
     if (!h->d_keymap) CU(cudaMalloc(&h->d_keymap, kMaxKeys));
     std::vector<uint8_t> present(kMaxKeys);

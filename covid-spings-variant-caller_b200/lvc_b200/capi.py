@@ -60,6 +60,10 @@ class ConsensusStats(C.Structure):
 
 assert C.sizeof(ConsensusStats) == 128
 
+# lvc_insertion (include/lvc.h): anchor position, length (0 = unresolved), 2-bit codes (base k in bits 2k), reads, depth
+INSERTION_DTYPE = np.dtype([("pos", "<i4"), ("len", "<u4"), ("seq", "<u8"), ("count", "<u4"), ("depth", "<u4")])
+assert INSERTION_DTYPE.itemsize == 24
+
 _lib: Optional[C.CDLL] = None
 
 # every symbol include/lvc.h declares: (name, restype, argtypes)
@@ -110,6 +114,10 @@ SIGNATURES = [
     ("lvc_copy_dense", C.c_int, [_H, C.c_void_p, C.c_void_p, C.c_void_p]),
     ("lvc_consensus", C.c_int, [_H, C.c_int64, C.c_int64, C.c_uint64, C.c_double, C.c_void_p, C.c_int, C.c_void_p,
                                 C.POINTER(ConsensusStats)]),
+    ("lvc_enable_insertions", C.c_int, [_H, C.c_uint32]),
+    ("lvc_copy_insertions", C.c_int, [_H, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]),
+    ("lvc_insertion_calls", C.c_int, [_H, C.c_int64, C.c_int64, C.c_uint64, C.c_double, C.c_void_p, C.c_uint32,
+                                      C.POINTER(C.c_uint32)]),
     ("lvc_num_planes", C.c_int, [_H]),
     ("lvc_plane_keys", C.c_int, [_H, C.c_void_p]),
     ("lvc_ensure_plane", C.c_int, [_H, C.c_uint16]),
@@ -574,6 +582,31 @@ class Handle:
         out = {name: int(getattr(st, name)) for name in CONSENSUS_COUNTERS}
         out["depth_ge"] = [int(st.depth_ge[i]) for i in range(min(thr.size, 8))]
         return seq[:n].tobytes(), out
+
+    # ---- insertions in the consensus
+    def enable_insertions(self, max_keys: int = 1 << 20):
+        """lvc_enable_insertions: count insertions from the next push on (only on empty tables)"""
+        self._check(self.lib.lvc_enable_insertions(self.h, int(max_keys)))
+
+    def _insertion_query(self, call) -> np.ndarray:
+        cap, n = 1 << 12, C.c_uint32(0)
+        while True:
+            out = np.zeros(cap, dtype=INSERTION_DTYPE)
+            self._check(call(out.ctypes.data, cap, C.byref(n)))
+            if n.value <= cap:
+                return out[:n.value]
+            cap = n.value
+
+    def copy_insertions(self) -> np.ndarray:
+        """every counted key (INSERTION_DTYPE, depth 0), sorted by (pos, len, seq)"""
+        return self._insertion_query(lambda out, cap, n: self.lib.lvc_copy_insertions(self.h, out, cap, n))
+
+    def insertion_calls(self, min_depth: int, threshold: float, p0: int = 0, p1: int = -1) -> np.ndarray:
+        """lvc_insertion_calls over [p0, p1) (p1 < 0: the whole contig): the called insertions, sorted by position"""
+        if int(min_depth) < 0:
+            raise ValueError(f"min_depth must be >= 0, not {min_depth}")
+        return self._insertion_query(lambda out, cap, n: self.lib.lvc_insertion_calls(
+            self.h, int(p0), int(p1), int(min_depth), float(threshold), out, cap, n))
 
     # ---- tables
     def plane_keys(self) -> np.ndarray:

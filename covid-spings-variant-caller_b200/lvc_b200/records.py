@@ -107,3 +107,21 @@ def format_consensus_fasta(contig: str, consensus: str, width: int = 60) -> str:
     letters per line."""
     seq = consensus.replace("-", "")
     return f">{contig}\n" + "".join(seq[i:i + width] + "\n" for i in range(0, len(seq), width))
+
+
+def decode_insertion(seq: int, length: int) -> str:
+    """lvc_insertion.seq (2-bit codes A, C, G, T = 0..3, base k in bits 2k) -> the inserted bases"""
+    return "".join("ACGT"[(int(seq) >> (2 * k)) & 3] for k in range(int(length)))
+
+
+def splice_insertions(consensus: str, calls) -> str:
+    """`consensus` (one letter per reference position) with each called insertion (INSERTION_DTYPE rows, positions
+    relative to the consensus's first letter) placed after the letter of its anchor"""
+    out, last = [], 0
+    for c in sorted(calls, key=lambda c: int(c["pos"])):
+        p = int(c["pos"]) + 1
+        out.append(consensus[last:p])
+        out.append(decode_insertion(c["seq"], c["len"]))
+        last = p
+    out.append(consensus[last:])
+    return "".join(out)

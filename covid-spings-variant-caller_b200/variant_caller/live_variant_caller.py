@@ -58,7 +58,8 @@ def _default_device() -> int:
 class LiveVariantCaller:
     def __init__(self, referenceFasta: str, minBaseQuality: int, minMappingQuality: int, minTotalDepth: int,
                  minAlleleDepth: int, minEvidenceRatio: float, maxVariants: int, device: Optional[int] = None,
-                 maxDepth: int = capi.MAX_DEPTH_DEFAULT, ignoreOverlaps: bool = True, overlapModel: Optional[str] = None):
+                 maxDepth: int = capi.MAX_DEPTH_DEFAULT, ignoreOverlaps: bool = True, overlapModel: Optional[str] = None,
+                 countInsertions: bool = False, maxInsertionKeys: int = 1 << 20):
         self.minBaseQuality = minBaseQuality
         self.minMappingQuality = minMappingQuality
         self.minTotalDepth = minTotalDepth
@@ -69,6 +70,10 @@ class LiveVariantCaller:
         # pysam's pileup(ignore_overlaps=True) default: htslib rewrites the qualities of overlapping mates.  The rule
         # changed between htslib releases and the reference does not pin pysam: "htslib-1.13" (default) or "htslib-1.10"
         self.overlapModel = capi.overlap_model_id(overlapModel) if ignoreOverlaps else capi.OVERLAP_OFF
+        # insertions for consensus(insertions=True) (include/lvc.h lvc_enable_insertions): a device hash table of at least
+        # maxInsertionKeys keys; records, VCF, memory and checkpoints never contain insertions
+        self.countInsertions = bool(countInsertions)
+        self.maxInsertionKeys = int(maxInsertionKeys)
         self.fastaFile = samio.Fasta(referenceFasta)
         self._device = _default_device() if device is None else device
         self._lock = threading.RLock()                      # the reference's callers use bare threads
@@ -89,6 +94,8 @@ class LiveVariantCaller:
         self._ref = self.fastaFile.fetch(reference=name)
         self._handle = capi.Handle(self._ref.encode("latin-1"), max(0, int(self.minBaseQuality)),
                                    int(self.minMappingQuality), self._device)
+        if self.countInsertions:
+            self._handle.enable_insertions(self.maxInsertionKeys)
 
     def close(self):
         with self._lock:
@@ -165,18 +172,38 @@ class LiveVariantCaller:
             fh.write(records.format_site_csv(depth, ad, self._ref))
 
     # ------------------------------------------------------------------ consensus + coverage (not in the reference API)
-    def consensus(self, minDepth: int = 10, threshold: float = 0.0) -> str:
+    def _insertion_calls(self, minDepth, threshold):
+        if not self.countInsertions:
+            raise ValueError("this LiveVariantCaller does not count insertions: construct it with countInsertions=True")
+        return self._handle.insertion_calls(int(minDepth), float(threshold))
+
+    def consensus(self, minDepth: int = 10, threshold: float = 0.0, insertions: bool = False) -> str:
         """Consensus genome, one letter per reference position (include/lvc.h lvc_consensus): 'N' below minDepth, '-'
         where deletions are the majority, IUPAC codes where the bases needed to reach `threshold` of the depth differ.
-        Computed on the device from the count tables; contains no insertions (they are not counted)."""
+        Computed on the device from the count tables.  It contains no insertions unless `insertions` is True, which needs a
+        caller constructed with countInsertions=True: then each called insertion (insertion_calls) follows the letter of
+        its anchor, uppercase.  After load_checkpoint, or with more distinct insertions than the table holds, that raises
+        (capi.LvcError) until reset_memory: the insertion counts do not cover the loaded tables."""
         with self._lock:
             seq, _ = self._handle.consensus(int(minDepth), float(threshold))
-        return seq.decode("ascii")
+            text = seq.decode("ascii")
+            if insertions:
+                text = records.splice_insertions(text, self._insertion_calls(minDepth, threshold))
+        return text
 
-    def write_consensus(self, outputFasta: str, minDepth: int = 10, threshold: float = 0.0):
+    def insertion_calls(self, minDepth: int = 10, threshold: float = 0.0) -> List[dict]:
+        """The insertions consensus(insertions=True) splices in (include/lvc.h lvc_insertion_calls), ascending position:
+        [{"pos": anchor (0-based; the insertion follows this reference base), "seq": inserted bases, "count": reads
+        carrying it, "depth": consensus depth at pos}].  Needs countInsertions=True; raises as consensus(insertions=True)."""
+        with self._lock:
+            calls = self._insertion_calls(minDepth, threshold)
+        return [{"pos": int(c["pos"]), "seq": records.decode_insertion(c["seq"], c["len"]), "count": int(c["count"]),
+                 "depth": int(c["depth"])} for c in calls]
+
+    def write_consensus(self, outputFasta: str, minDepth: int = 10, threshold: float = 0.0, insertions: bool = False):
         """FASTA of `consensus()` with the deletion calls removed, 60 letters per line."""
         with self._lock:
-            text = records.format_consensus_fasta(self._contig, self.consensus(minDepth, threshold))
+            text = records.format_consensus_fasta(self._contig, self.consensus(minDepth, threshold, insertions))
         with open(outputFasta, "w") as fh:
             fh.write(text)
 

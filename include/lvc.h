@@ -279,7 +279,8 @@ int lvc_copy_dense(lvc_handle* h, uint32_t* depth /*[G]*/, uint32_t* ad /*[G*4] 
  *   else "=ACMGRSVTWYHKDBN"[mask], mask = OR of (1 << rank) of the taken bases (A=1 C=2 G=4 T=8: the BAM nibble
  *   alphabet is the IUPAC code of the mask; a deletion taken later is not in the mask).
  * threshold 0 is a plain majority call; 0.5-0.75 gives mixed positions ambiguity codes.  Letters are uppercase.
- * Insertions are not in the tables, so the consensus contains none.
+ * Insertions are not in these tables, so the letters contain none; unless counting is enabled (lvc_enable_insertions
+ * below), the consensus has no insertions.
  * Statistics over the same range: n_positions, depth_sum, depth_max, n_low_depth (d < min_depth), n_N (every 'N'),
  * n_deleted (every '-'), n_ambiguous (two- and three-base codes), n_mismatch (a single-base call other than the reference
  * letter, where toupper(ref[p]) is A/C/G/T), depth_ge[i] (d >= depth_thresholds[i], i < n_thresholds; the rest 0).
@@ -294,6 +295,48 @@ typedef struct lvc_consensus_stats {
 } lvc_consensus_stats;                                                   /* 128 bytes */
 int lvc_consensus(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, double threshold,
                   const uint32_t* depth_thresholds, int n_thresholds, uint8_t* seq_out, lvc_consensus_stats* stats_out);
+
+/* ---- insertions in the consensus genome [EXT] ---------------------------------------------------
+ * Opt-in: records, VCF, `memory` and checkpoints never contain insertions (the reference emits none), and nothing that
+ * exists changes while counting is on, except that each push launches one more kernel.
+ * Counting rule.  A read the deposit walks (it passes read_passes_filter, has a reference-consuming op and lies inside
+ * [0, G); reads skipped with LVC_ERANGE count nothing) counts each I op that meets all of:
+ *   - the op before it, ignoring P ops and ops of length 0, is a match op (M, =, X); an I op after S, D or N, or at the
+ *     start of the read, is not counted.  [EXT] htslib also reports insertions on deletion anchors; this rule does not;
+ *   - the anchor -- the last base of that match op, at reference position p -- has quality >= min_base_quality (the
+ *     pileup entry on which htslib reports indel > 0 and which pysam's base-quality filter keeps).
+ * Key: (p, len, seq) when len <= 32 and every inserted base is A/C/G/T with quality >= min_base_quality (seq = 2-bit
+ * codes A,C,G,T = 0..3, base k in bits 2k); otherwise (p, 0, 0), an "unresolved" insertion that counts towards the
+ * insertions at p but is never emitted.  The counts are the same for every batch form (byte or 2-bit qualities, 4-bit
+ * bases or 2-bit base codes): the rule never needs a base below the threshold.  Mate-overlap rewrites need no special
+ * case: the qualities are read as the batch carries them.  Once per batch, in a device hash table.
+ * lvc_enable_insertions  only on empty tables (after lvc_create or lvc_reset, before any push or import), else
+ *                        LVC_EINVAL; refused with peer tables attached (and lvc_peer_attach is refused on a handle that
+ *                        counts).  The table has at least 2 * max_keys slots (a power of two); it holds at least
+ *                        max_keys keys, and a key is dropped only when every slot holds another.  lvc_reset clears it and
+ *                        keeps counting on.  Timer 4 of lvc_get_timing times the counting kernel.
+ * Both queries fail with LVC_EINVAL after lvc_import_plane / _dels / _covdiff / _first or lvc_reduce_tables (the tables
+ * then hold counts the insertion table does not cover) until lvc_reset, and with LVC_ENOMEM (the message gives the number)
+ * if keys were dropped.  *n_out > cap: call again with a larger buffer.
+ * lvc_copy_insertions    every key with its count (depth = 0), sorted by (pos, len, seq).
+ * lvc_insertion_calls    for each anchor p in [p0, p1) (p1 < 0: the whole contig; arguments checked as lvc_consensus):
+ *                        d = the consensus depth of p, I = the sum of every count at p (unresolved included),
+ *                        none = d - I.  The resolved key s is emitted (count, depth = d) iff the consensus letter of p for
+ *                        (min_depth, threshold) is neither 'N' nor '-', count(s) > none, count(s) > the unresolved count,
+ *                        count(s) > every other resolved count at p, and count(s) / d >= threshold (fp64 division).
+ *                        Every comparison is strict: a tie emits nothing.  Sorted by pos (at most one per position).
+ * The splice: a called sequence follows the letter of its anchor. */
+typedef struct lvc_insertion {
+    int32_t pos;        /* anchor: 0-based position of the reference base the insertion follows */
+    uint32_t len;       /* inserted bases; 0 = unresolved */
+    uint64_t seq;       /* 2-bit codes A,C,G,T = 0..3, base k in bits 2k */
+    uint32_t count;     /* reads carrying the key */
+    uint32_t depth;     /* lvc_insertion_calls: consensus depth at pos; lvc_copy_insertions: 0 */
+} lvc_insertion;        /* 24 bytes */
+int lvc_enable_insertions(lvc_handle* h, uint32_t max_keys);
+int lvc_copy_insertions(lvc_handle* h, lvc_insertion* out, uint32_t cap, uint32_t* n_out);
+int lvc_insertion_calls(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, double threshold,
+                        lvc_insertion* out, uint32_t cap, uint32_t* n_out);
 
 /* ---- table access: self.memory (live_variant_caller.py:31), checkpoints (:40-52), tests, NCCL ----
  * A "plane" holds, for one (allele group, quality) key, uint32 counts [G][4].  key = group<<8 | q;
@@ -372,7 +415,8 @@ uint64_t lvc_launch_count(lvc_handle* h);
  * host admission dropped are never shipped */
 uint64_t lvc_h2d_payload_bytes(lvc_handle* h);
 /* per-kernel device time from CUDA events recorded on the handle's stream around every launch while
- * timing is on.  which: 0 = tiled deposit, 1 = general deposit, 2 = genotype, 3 = consensus.  Reading resets. */
+ * timing is on.  which: 0 = tiled deposit, 1 = general deposit, 2 = genotype, 3 = consensus, 4 = insertion counts (only
+ * on a handle that counts them, lvc_enable_insertions).  Reading resets. */
 int lvc_set_timing(lvc_handle* h, int on);
 int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launches);
 int lvc_version(void);
