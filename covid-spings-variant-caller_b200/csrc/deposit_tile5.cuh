@@ -50,14 +50,15 @@ constexpr int kTile5CtasPerSM = LVC5_CTAS_PER_SM;
 #endif
 constexpr int kTask5Runs = 224;                  // runs per task: 7 units per lane, three bit planes hold <= 7
 
+// Run table: per run only what the task table and the pass loop need -- the read's start column (s_rs), the packed
+// (start column, key offset | length) record (s_pk) and (window << 8 | read index) (s_rix).  The cold-path deposit, the
+// first-seen scan and multi-window chunks derive a run's column, length and payload offset from s_pk: inside one staged
+// window a run's payload offset is w_rel + (s_pk.y & 0xFFFF).
 struct Tile5Smem {
     static constexpr uint32_t key_off = 0;                                     // 4-bit keys, little-endian nibble order
     static constexpr uint32_t key_bytes = kSlack + kT5KeyCapBases / 2 + 32 + kSlack;
-    static constexpr uint32_t pos_off = key_off + key_bytes;                   // i32 [kMaxRuns]
-    static constexpr uint32_t qo_off = pos_off + kMaxRuns * 4;                 // u32 [kMaxRuns]
-    static constexpr uint32_t len_off = qo_off + kMaxRuns * 4;                 // u16 [kMaxRuns]
-    static constexpr uint32_t rd_off = len_off + kMaxRuns * 2;                 // u16 [kMaxRuns]
-    static constexpr uint32_t rix_off = rd_off + kMaxRuns * 2;                 // u16 [kMaxRuns]
+    static constexpr uint32_t rs_off = key_off + key_bytes;                    // i32 [kMaxRuns] start column of the run's read
+    static constexpr uint32_t rix_off = rs_off + kMaxRuns * 4;                 // u16 [kMaxRuns]
     static constexpr uint32_t dlist_off = rix_off + kMaxRuns * 2;              // u16 [kT5Reads]
     static constexpr uint32_t slab_a_off = dlist_off + kT5Reads * 2;         // u32 [kMaxSlabs]
     static constexpr uint32_t slab_pre_off = slab_a_off + kMaxSlabs * 4;       // u32 [kMaxSlabs+1]
@@ -72,6 +73,20 @@ struct Tile5Smem {
 };
 constexpr size_t kTile5SmemBytes = Tile5Smem::total;
 static_assert((kTile5SmemBytes + 1024) * kTile5CtasPerSM <= 227 * 1024, "the intended CTAs per SM must fit");
+
+// Phase clocks (build with -DLVC5_PHASE_CLOCKS; tools/bench_phases.py reads them through lvc_phase_clocks): thread 0
+// of every CTA of the last launch records its SM and clock64() at the phase boundaries below (0 = not reached).
+#ifdef LVC5_PHASE_CLOCKS
+enum { T5P_ENTRY, T5P_HEADERS, T5P_EXTENTS, T5P_BARRIER_A, T5P_BARRIER_B, T5P_BARRIER_C, T5P_TASKS_END, T5P_EXIT, T5P_N };
+constexpr uint32_t kT5PhaseMaxCtas = 1u << 16;
+__device__ unsigned long long g_t5_phase[kT5PhaseMaxCtas][1 + T5P_N];     // [cta] = smid, stamps
+#define T5_STAMP(k)                                                                                        \
+    do {                                                                                                   \
+        if (threadIdx.x == 0 && blockIdx.x < kT5PhaseMaxCtas) g_t5_phase[blockIdx.x][1 + (k)] = clock64(); \
+    } while (0)
+#else
+#define T5_STAMP(k) do {} while (0)
+#endif
 
 __device__ __forceinline__ uint32_t lop3_xor3(uint32_t a, uint32_t b, uint32_t c) {
     uint32_t d;
@@ -116,10 +131,7 @@ __global__ void __launch_bounds__(kT5Threads, kTile5CtasPerSM)
 k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp, LVC_GC TileParams tp) {
     extern __shared__ __align__(128) unsigned char smem[];
     const uint32_t sbase = smem_u32(smem);
-    int32_t* s_pos = reinterpret_cast<int32_t*>(smem + Tile5Smem::pos_off);
-    uint32_t* s_qo = reinterpret_cast<uint32_t*>(smem + Tile5Smem::qo_off);
-    uint16_t* s_len = reinterpret_cast<uint16_t*>(smem + Tile5Smem::len_off);
-    uint16_t* s_rd = reinterpret_cast<uint16_t*>(smem + Tile5Smem::rd_off);
+    int32_t* s_rs = reinterpret_cast<int32_t*>(smem + Tile5Smem::rs_off);
     uint16_t* s_rix = reinterpret_cast<uint16_t*>(smem + Tile5Smem::rix_off);
     uint16_t* s_dlist = reinterpret_cast<uint16_t*>(smem + Tile5Smem::dlist_off);
     uint32_t* s_slab_a = reinterpret_cast<uint32_t*>(smem + Tile5Smem::slab_a_off);
@@ -138,6 +150,15 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
     // grid drains; it still waits for this grid's completion before reading
     asm volatile("griddepcontrol.launch_dependents;");
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+#ifdef LVC5_PHASE_CLOCKS
+    if (tid == 0 && blockIdx.x < kT5PhaseMaxCtas) {
+        uint32_t smid;
+        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+        g_t5_phase[blockIdx.x][0] = smid;
+        for (int k = 1; k < T5P_N; ++k) g_t5_phase[blockIdx.x][1 + k] = 0;
+    }
+    T5_STAMP(T5P_ENTRY);
+#endif
     const uint32_t qprim4 = tp.qprim * 0x01010101u;
     const int mbq = dp.min_bq < 1 ? 1 : (dp.min_bq > 128 ? 128 : dp.min_bq);
     const uint32_t ge_add4 = (uint32_t)(0x80 - mbq) * 0x01010101u;
@@ -158,7 +179,7 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
     }
     // a chunk in which the host admission (htslib max_depth) dropped every read ends here, after ONE load per thread:
     // nothing else of its headers is waited for
-    if (!__syncthreads_or(hd.keep & 1u)) return;
+    if (!__syncthreads_or(hd.keep & 1u)) { T5_STAMP(T5P_EXIT); return; }
     if (b.hdr_lazy) hdr_load1<kT5Reads>(b, cur, tid, hd, so0);
     if (tid < 66) {
         // edge masks of a 32-column unit, one nibble per column: [0][n] keeps the columns >= n, [1][n] the columns < n
@@ -174,7 +195,8 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
     }
     hdr_load2(b, hd, dp.min_mq);       // CIGAR ops, only for reads that pass the read-level filter
     // a chunk in which no read passes the read-level filter ends here
-    if (!__syncthreads_or(read_passes_filter(hd.flag, hd.mapq, hd.keep, dp.min_mq))) return;
+    if (!__syncthreads_or(read_passes_filter(hd.flag, hd.mapq, hd.keep, dp.min_mq))) { T5_STAMP(T5P_EXIT); return; }
+    T5_STAMP(T5P_HEADERS);
     // Up to here only the batch was read.  The tables may still be in use by the previous kernel of the stream (this
     // kernel is launched with programmatic stream serialization): wait for it before the first table access.
 #if LVC5_WAIT == 0
@@ -196,6 +218,7 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
         if (lane == 0 && hi) { atomicMin(&sc[0], lo); atomicMax(&sc[1], hi); }
     }
     __syncthreads();
+    T5_STAMP(T5P_EXTENTS);
     const uint32_t min_rel = sc[0], max_rel = sc[1];
     if (max_rel == 0) {
         // no read of this chunk can take the tiled path: hand over what must be deposited and leave
@@ -208,30 +231,27 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
         const uint32_t n_def = s_misc[6];
         asm volatile("griddepcontrol.wait;" ::: "memory");
         for (uint32_t d = warp; d < n_def; d += kT5Warps) (PEER ? deposit_read_warp_peer : deposit_read_warp)(b, tv, dp, cur * kT5Reads + s_dlist[d], lane);
+        T5_STAMP(T5P_EXIT);
         return;
     }
     // staging base: 16-byte aligned start of the first such read
     const uint64_t base_abs = (so0 + min_rel) & ~15ull;
+    const uint32_t base_rel = (uint32_t)(base_abs - so0);            // may wrap below zero: used mod 2^32
 #ifndef LVC5_NO_PREFETCH
     {
         // ask L2 for the chunk's payload now: classification and the run table hide the DRAM latency of the staging
-        // loads (measured on config 5: 0.524 -> 0.498 ms)
-        const uint64_t q0 = base_abs, q1 = so0 + max_rel;
-        if (QC) {
-            for (uint64_t a = (q0 >> 2) + (uint64_t)tid * 128u; a < ((q1 + 3) >> 2); a += (uint64_t)kT5Threads * 128u)
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(b.qual + a));
-        } else
-        for (uint64_t a = q0 + (uint64_t)tid * 128u; a < q1; a += (uint64_t)kT5Threads * 128u)
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(b.qual + a));
-        if (B2) {
-            for (uint64_t a = (q0 >> 2) + (uint64_t)tid * 128u; a < ((q1 + 3) >> 2); a += (uint64_t)kT5Threads * 128u)
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(b.seq4 + a));
-        } else
-        for (uint64_t a = (q0 >> 1) + (uint64_t)tid * 128u; a < ((q1 + 1) >> 1); a += (uint64_t)kT5Threads * 128u)
-            asm volatile("prefetch.global.L2 [%0];" ::"l"(b.seq4 + a));
+        // loads (measured on config 5: 0.524 -> 0.498 ms).  The 128-byte lines of the quality array, then those of the
+        // base array, numbered from the (16-base aligned) staging base: one line per thread for a chunk of short reads
+        const uint32_t span = max_rel - base_rel;                    // bases from the staging base to the last read's end
+        constexpr int qsh = QC ? 2 : 0, ssh = B2 ? 2 : 1;            // log2 bases per byte
+        const uint32_t nq = (((span + (1u << qsh) - 1u) >> qsh) + 127u) >> 7;
+        const uint32_t ns = (((span + (1u << ssh) - 1u) >> ssh) + 127u) >> 7;
+        const uint8_t* pq = b.qual + (base_abs >> qsh);
+        const uint8_t* ps = b.seq4 + (base_abs >> ssh);
+        for (uint32_t l = (uint32_t)tid; l < nq + ns; l += kT5Threads)
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(l < nq ? pq + 128u * l : ps + 128u * (l - nq)));
     }
 #endif
-    const uint32_t base_rel = (uint32_t)(base_abs - so0);            // may wrap below zero: used mod 2^32
     {
         const uint32_t chunk0 = cur * kT5Reads;
         // ---- (2) classify this thread's read: filter, match runs, deletion entries
@@ -384,6 +404,7 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
             }
         }
         __syncthreads();                                                   // barrier A
+        T5_STAMP(T5P_BARRIER_A);
         uint32_t n_runs = 0, my_base = 0;
 #pragma unroll
         for (int w = 0; w < kT5Warps; ++w) {
@@ -456,10 +477,7 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
                 for (int k = 0; k < kMaxRunsPerRead; ++k) {
                     if ((uint32_t)k < nr) {
                         const uint32_t idx = idx0 + k;
-                        s_pos[idx] = run_pos[k];
-                        s_qo[idx] = off + run_q[k];
-                        s_len[idx] = (uint16_t)run_len[k];
-                        s_rd[idx] = (uint16_t)(run_pos[k] - hd.pos);
+                        s_rs[idx] = hd.pos;
                         s_rix[idx] = (uint16_t)((win << 8) | (uint32_t)tid);
                         // (start column, key offset inside the read's window | length << 16): one 8-byte load per unit
                         s_pk[idx] = make_uint2((uint32_t)run_pos[k], ((off + run_q[k] - win * kT5WinStride) & 0xFFFFu) | (run_len[k] << 16));
@@ -467,6 +485,7 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
                 }
             }
             __syncthreads();                                               // barrier B: run table visible
+            T5_STAMP(T5P_BARRIER_B);
         }
 
         // ---- (5) staged windows of runs (one per chunk unless reads are long)
@@ -484,41 +503,40 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
                 const uint32_t w_rel = win * kT5WinStride;                   // window start relative to the base
                 const uint64_t qbeg = base_abs + w_rel;                    // 16-byte aligned
                 // column range of these runs
-                const int32_t cmin = s_pos[a0] - (int32_t)s_rd[a0];
+                const int32_t cmin = s_rs[a0];
                 int32_t cmax = chunk_cmax;                                 // chunk-wide (an upper bound for any window)
                 if (n_win > 1) {                                           // long reads: exact range of this window's runs
                     __syncthreads();
                     if (tid == 0) s_misc[4] = 0;
                     __syncthreads();
                     int32_t e = 0;
-                    for (uint32_t r = a0 + tid; r < a1; r += kT5Threads) e = max(e, s_pos[r] + (int32_t)s_len[r]);
+                    for (uint32_t r = a0 + tid; r < a1; r += kT5Threads) e = max(e, (int32_t)s_pk[r].x + (int32_t)(s_pk[r].y >> 16));
                     e = __reduce_max_sync(0xFFFFFFFFu, e);
                     if (lane == 0 && e) atomicMax(reinterpret_cast<int32_t*>(&s_misc[4]), e);
                     __syncthreads();
                     cmax = (int32_t)s_misc[4];
                 }
-                // Task table of one column window: per 32-column slab the candidate run range (binary search over the
-                // sorted read start of each run) and the exclusive scan of the task counts.  One warp does it.  For the
-                // first column window that happens while the warp's first payload loads are in flight.
+                // Task table of one column window: per 32-column slab the candidate run range and the exclusive scan of
+                // the task counts.  One warp does it, before its share of the staging, and the other warps wait for it at
+                // barrier C, so the two lower bounds of a slab over the read starts of the runs (non-decreasing: a batch is
+                // coordinate sorted) are independent searches on two lanes: lane s finds the end of slab s's range (the
+                // first run whose read starts at or after the slab's end), lane 8 + s its first run (the first run whose
+                // read starts after slab start - max span).  Half the chain of dependent shared loads of one lane doing both.
                 auto slab_setup = [&](int32_t wc0) {
                     const int nslab = min(kMaxSlabs, (cmax - wc0 + kSlabCols - 1) / kSlabCols);
                     uint32_t cnt = 0, first_run = 0;
-                    if (lane < nslab) {
-                        const int32_t s_lo = wc0 + lane * kSlabCols, s_hi = s_lo + kSlabCols;
-                        uint32_t lo = a0, hi = a1;               // first run whose read starts at or after s_hi
+                    {
+                        static_assert(kMaxSlabs == 8, "two searches per slab on lanes s and 8 + s");
+                        const int sl = lane & 15;
+                        const int32_t s_lo = wc0 + (sl & 7) * kSlabCols;
+                        const int64_t thr = sl < 8 ? (int64_t)s_lo + kSlabCols - 1 : (int64_t)s_lo - (int64_t)maxspan;
+                        uint32_t lo = a0, hi = a1;               // first run whose read starts after thr
                         while (lo < hi) {
                             const uint32_t m = (lo + hi) >> 1;
-                            if (s_pos[m] - (int32_t)s_rd[m] < s_hi) lo = m + 1; else hi = m;
+                            if ((int64_t)s_rs[m] <= thr) lo = m + 1; else hi = m;
                         }
-                        const uint32_t bnd = lo;
-                        const int64_t thr = (int64_t)s_lo - (int64_t)maxspan;   // first run whose read starts after thr
-                        lo = a0; hi = bnd;
-                        while (lo < hi) {
-                            const uint32_t m = (lo + hi) >> 1;
-                            if ((int64_t)(s_pos[m] - (int32_t)s_rd[m]) <= thr) lo = m + 1; else hi = m;
-                        }
-                        first_run = lo;
-                        cnt = bnd - lo;
+                        const uint32_t fr = __shfl_down_sync(0xFFFFFFFFu, lo, 8);
+                        if (lane < nslab) { first_run = fr; cnt = lo - fr; }
                     }
                     // tasks of a slab are equal shares of its candidate runs, <= kTask5Runs each (whole passes of 32)
                     const uint32_t groups = (cnt + kTask5Runs - 1) / kTask5Runs;
@@ -574,16 +592,17 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
                                 while (m80) {
                                     const int bb = (__ffs(m80) - 1) >> 3;
                                     m80 &= ~(0x80u << (8 * bb));
-                                    const uint32_t x_rel = w_rel + 16u * gg + 4u * (uint32_t)w + (uint32_t)bb;
-                                    uint32_t lo = a0, hi = a1;             // last run with s_qo <= x_rel
-                                    while (lo < hi) { const uint32_t m = (lo + hi) >> 1; if (s_qo[m] <= x_rel) lo = m + 1; else hi = m; }
+                                    const uint32_t x_win = 16u * gg + 4u * (uint32_t)w + (uint32_t)bb;
+                                    uint32_t lo = a0, hi = a1;             // last run whose payload starts at or before x_win
+                                    while (lo < hi) { const uint32_t m = (lo + hi) >> 1; if ((s_pk[m].y & 0xFFFFu) <= x_win) lo = m + 1; else hi = m; }
                                     if (lo > a0) {
-                                        const uint32_t r = lo - 1, d = x_rel - s_qo[r];
+                                        const uint2 pk = s_pk[lo - 1];
+                                        const uint32_t r = lo - 1, d = x_win - (pk.y & 0xFFFFu);
 #if LVC5_WAIT == 2
                                         asm volatile("griddepcontrol.wait;" ::: "memory");
 #endif
-                                        if (d < (uint32_t)s_len[r])
-                                            deposit_base<PEER>(tv, dp, (int64_t)s_pos[r] + d, (sx >> (4 * bb)) & 15u,
+                                        if (d < (pk.y >> 16))
+                                            deposit_base<PEER>(tv, dp, (int64_t)(int32_t)pk.x + d, (sx >> (4 * bb)) & 15u,
                                                          (qv >> (8 * bb)) & 255u, chunk_ord + (s_rix[r] & 255u));
                                     }
                                 }
@@ -610,16 +629,17 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
                             while (cold) {
                                 const uint32_t bb = (uint32_t)(__ffs(cold) - 1) >> 1;          // base 0..15 of the group
                                 cold &= cold - 1;
-                                const uint32_t x_rel = w_rel + 16u * gg + bb;
-                                uint32_t lo = a0, hi = a1;             // last run with s_qo <= x_rel
-                                while (lo < hi) { const uint32_t m = (lo + hi) >> 1; if (s_qo[m] <= x_rel) lo = m + 1; else hi = m; }
+                                const uint32_t x_win = 16u * gg + bb;
+                                uint32_t lo = a0, hi = a1;             // last run whose payload starts at or before x_win
+                                while (lo < hi) { const uint32_t m = (lo + hi) >> 1; if ((s_pk[m].y & 0xFFFFu) <= x_win) lo = m + 1; else hi = m; }
                                 if (lo > a0) {
-                                    const uint32_t r = lo - 1, d = x_rel - s_qo[r];
+                                    const uint2 pk = s_pk[lo - 1];
+                                    const uint32_t r = lo - 1, d = x_win - (pk.y & 0xFFFFu);
 #if LVC5_WAIT == 2
                                     asm volatile("griddepcontrol.wait;" ::: "memory");
 #endif
-                                    if (d < (uint32_t)s_len[r])
-                                        deposit_base<PEER>(tv, dp, (int64_t)s_pos[r] + d, ((bb < 8u ? s0 : s1) >> (4u * (bb & 7u))) & 15u,
+                                    if (d < (pk.y >> 16))
+                                        deposit_base<PEER>(tv, dp, (int64_t)(int32_t)pk.x + d, ((bb < 8u ? s0 : s1) >> (4u * (bb & 7u))) & 15u,
                                                            (b.qdict >> (8u * ((w >> (2u * bb)) & 3u))) & 255u, chunk_ord + (s_rix[r] & 255u));
                                 }
                             }
@@ -683,6 +703,7 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
                         if (warp == 0) slab_setup(wc0);
                     }
                     __syncthreads();                                       // barrier C: keys staged, task table built
+                    T5_STAMP(T5P_BARRIER_C);
                     const uint32_t n_tasks = s_slab_pre[nslab];
 
                     // ---- tasks: (slab of 32 columns, share of its candidate runs); lane = one run per pass, all 32 columns
@@ -831,9 +852,10 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
                                         const uint32_t r = q0 + (uint32_t)lane;
                                         bool hit = false;
                                         if (r < se) {
-                                            const int32_t jj = icol - s_pos[r];
-                                            if (jj >= 0 && jj < (int32_t)s_len[r]) {
-                                                const uint32_t kk = (s_qo[r] - w_rel) + (uint32_t)jj;
+                                            const uint2 pk = s_pk[r];
+                                            const int32_t jj = icol - (int32_t)pk.x;
+                                            if (jj >= 0 && jj < (int32_t)(pk.y >> 16)) {
+                                                const uint32_t kk = (pk.y & 0xFFFFu) + (uint32_t)jj;
                                                 const uint32_t key = (lds32(k_smem + ((kk >> 3) << 2)) >> ((kk & 7u) * 4u)) & 15u;
                                                 hit = key == want;
                                             }
@@ -860,9 +882,11 @@ k_deposit_tile5(LVC_GC BatchView b, LVC_GC TableView tv, LVC_GC DepositParams dp
 #endif
         // ---- reads the tiled path could not take (many runs, long, exotic base codes): general path, one warp each
         __syncthreads();
+        T5_STAMP(T5P_TASKS_END);
         const uint32_t n_def = s_misc[6];
         for (uint32_t d = warp; d < n_def; d += kT5Warps) (PEER ? deposit_read_warp_peer : deposit_read_warp)(b, tv, dp, chunk0 + s_dlist[d], lane);
     }
+    T5_STAMP(T5P_EXIT);
 }
 
 }  // namespace lvc

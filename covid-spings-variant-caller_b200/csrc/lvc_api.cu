@@ -1382,6 +1382,16 @@ void* lvc_first_devptr(lvc_handle* h, int group) {
 }
 uint64_t lvc_launch_count(lvc_handle* h) { return h ? h->launches : 0; }
 uint64_t lvc_h2d_payload_bytes(lvc_handle* h) { return h ? h->h2d_payload_bytes : 0; }
+#ifdef LVC5_PHASE_CLOCKS
+// phase-clock builds only: copies the per-CTA records of the last tiled launch (SM id, then T5P_N clock64() stamps per CTA)
+// to `out`, which holds `max_ctas` records; returns the number of records the build keeps, or -1 on a CUDA error
+int lvc_phase_clocks(void* out, uint32_t max_ctas) {
+    const size_t rec = sizeof(g_t5_phase[0]);
+    const size_t n = std::min<size_t>(max_ctas, kT5PhaseMaxCtas);
+    if (cudaDeviceSynchronize() != cudaSuccess || cudaMemcpyFromSymbol(out, g_t5_phase, n * rec) != cudaSuccess) return -1;
+    return (int)kT5PhaseMaxCtas;
+}
+#endif
 
 }  // extern "C"
 
