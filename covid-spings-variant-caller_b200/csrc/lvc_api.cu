@@ -1,5 +1,6 @@
 // liblvc_b200.so -- C-ABI (include/lvc.h) over the sm_100a kernels.  No torch types, no CPU fallback.
 #include <algorithm>
+#include <cctype>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -21,6 +22,7 @@
 #include "genotype.cuh"
 #include "consensus.cuh"
 #include "insertions.cuh"
+#include "linkage.cuh"
 #include "deposit_select.hpp"
 #include "overlap.hpp"
 #include "qcode.hpp"
@@ -120,10 +122,18 @@ struct lvc_handle {
     bool ins_uncovered = false;              // an import or reduction since lvc_reset: counts the insertion table lacks
     DevBuf i_list, i_scratch;
 
+    // variant linkage (lvc_set_linkage_sites): link.counts == nullptr while counting is off.  Host copies of the sites
+    // and of the pair offsets give lvc_copy_linkage its (a, b) order.
+    LinkTable link = {nullptr, nullptr, nullptr, 0};
+    uint64_t link_pairs = 0;
+    std::vector<int32_t> link_pos;
+    std::vector<uint8_t> link_alt;
+    std::vector<uint32_t> link_npart;        // partners after each site
+
     // optional per-kernel timing (CUDA events on the launching stream)
     bool timing = false;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[5];   // 0 tiled deposit, 1 general deposit, 2 genotype, 3 consensus,
-                                                              // 4 insertion counts
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[6];   // 0 tiled deposit, 1 general deposit, 2 genotype, 3 consensus,
+                                                              // 4 insertion counts, 5 linkage counts
     std::vector<cudaEvent_t> ev_pool;
 };
 
@@ -340,11 +350,12 @@ void lvc_destroy(lvc_handle* h) {
     cudaFree(h->d_first_arr); cudaFree(h->d_newkeys); cudaFree(h->d_replay); cudaFree(h->d_status); cudaFree(h->d_keymap);
     if (h->h_status) cudaFreeHost(h->h_status);
     if (h->h_sample) cudaFreeHost(h->h_sample);
-    for (int w = 0; w < 5; ++w) for (auto& pr : h->ev[w]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
+    for (int w = 0; w < 6; ++w) for (auto& pr : h->ev[w]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
     for (auto e : h->ev_pool) cudaEventDestroy(e);
     cudaFree(h->d_elut); cudaFree(h->d_out_depth); cudaFree(h->d_out_ad); cudaFree(h->d_out_lik);
     cudaFree(h->d_cand_count);
     cudaFree(h->ins.keys); cudaFree(h->ins.counts); cudaFree(h->ins.dropped);
+    cudaFree((void*)h->link.pos); cudaFree((void*)h->link.site); cudaFree(h->link.counts);
     for (DevBuf* b : {&h->b_pos, &h->b_flag, &h->b_mapq, &h->b_keep, &h->b_coff, &h->b_cig, &h->b_soff, &h->b_seq,
                       &h->b_qual, &h->g_order_ptrs, &h->g_order_keys, &h->g_cand, &h->g_pconst, &h->c_order_ptrs,
                       &h->c_seq, &h->c_stats, &h->i_list, &h->i_scratch})
@@ -395,6 +406,7 @@ int lvc_reset(lvc_handle* h) {
         CU(cudaMemsetAsync(h->ins.counts, 0, slots * sizeof(uint32_t), h->stream));
         CU(cudaMemsetAsync(h->ins.dropped, 0, sizeof(uint32_t), h->stream));
     }
+    if (h->link.counts) CU(cudaMemsetAsync(h->link.counts, 0, h->link_pairs * 9 * sizeof(uint32_t), h->stream));
     h->tables_touched = false;
     h->ins_uncovered = false;
     h->ordinal = 0;
@@ -547,6 +559,18 @@ static int launch_count_insertions(lvc_handle* h, const BatchView& bv) {
     return LVC_OK;
 }
 
+// The linkage counts of one batch (lvc_set_linkage_sites), launched like launch_count_insertions and behind it.
+static int launch_count_linkage(lvc_handle* h, const BatchView& bv) {
+    if (!h->link.counts || bv.n_reads == 0) return LVC_OK;
+    LinkCountParams cp;
+    cp.G = h->G; cp.min_bq = h->min_bq; cp.min_mq = h->min_mq;
+    { KernelTimer t(h, 5);
+      CU(launch_kernel(h, k_count_linkage, dim3((bv.n_reads + kLinkThreads - 1) / kLinkThreads), dim3(kLinkThreads), 0, true,
+                       bv, h->link, cp, bv.n_reads)); }
+    CU(cudaGetLastError());
+    return LVC_OK;
+}
+
 static int deposit_with_replay(lvc_handle* h, const BatchView& bv, uint64_t n_cigar_ops, uint64_t n_qual,
                                const lvc_batch* account = nullptr) {
     if ((uint64_t)h->ordinal + bv.n_reads >= 0xFFFFFFFFull)
@@ -556,6 +580,8 @@ static int deposit_with_replay(lvc_handle* h, const BatchView& bv, uint64_t n_ci
     int rc = launch_deposit(h, bv, 0, n_cigar_ops, n_qual);
     if (rc) return rc;
     rc = launch_count_insertions(h, bv);           // once per batch: the replay pass below does not count again
+    if (rc) return rc;
+    rc = launch_count_linkage(h, bv);
     if (rc) return rc;
     CU(cudaMemcpyAsync(h->h_status, h->d_status, ST_WORDS * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
     CU(cudaMemcpyAsync(h->h_status + ST_WORDS, h->d_newkeys, 32 * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
@@ -834,6 +860,8 @@ int lvc_push_batch_device_async(lvc_handle* h, const lvc_batch* b) {
     if (rc) return rc;
     rc = launch_count_insertions(h, bv);
     if (rc) return rc;
+    rc = launch_count_linkage(h, bv);
+    if (rc) return rc;
     h->ordinal += b->n_reads;
     return LVC_OK;
 }
@@ -860,8 +888,9 @@ int lvc_set_timing(lvc_handle* h, int on) {
 }
 
 int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launches) {
-    if (!h || which < 0 || which > 4 || !ms_total || !n_launches) return LVC_EINVAL;
+    if (!h || which < 0 || which > 5 || !ms_total || !n_launches) return LVC_EINVAL;
     if (which == 4 && !h->ins.keys) return fail(h, LVC_EINVAL, "timer 4 (insertion counts) needs lvc_enable_insertions");
+    if (which == 5 && !h->link.counts) return fail(h, LVC_EINVAL, "timer 5 (linkage counts) needs lvc_set_linkage_sites");
     CU(cudaSetDevice(h->device));
     CU(cudaStreamSynchronize(h->stream));
     double tot = 0.0;
@@ -1260,6 +1289,116 @@ int lvc_insertion_calls(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_dept
     CU(cudaStreamSynchronize(h->stream));
     *n_out = h->h_status[0];
     return copy_sorted(h, *n_out, out, cap);
+}
+
+// ------------------------------------------------------------------------------------------------
+// variant linkage
+// ------------------------------------------------------------------------------------------------
+static_assert(sizeof(lvc_linkage_pair) == 48, "lvc_linkage_pair layout");
+
+static void free_linkage(lvc_handle* h) {
+    cudaFree((void*)h->link.pos); cudaFree((void*)h->link.site); cudaFree(h->link.counts);
+    h->link = LinkTable{nullptr, nullptr, nullptr, 0};
+    h->link_pairs = 0;
+    h->link_pos.clear(); h->link_alt.clear(); h->link_npart.clear();
+}
+
+static uint8_t nibble_of(uint8_t c) {
+    switch (c) { case 'A': return 1; case 'C': return 2; case 'G': return 4; case 'T': return 8; default: return 0; }
+}
+
+int lvc_set_linkage_sites(lvc_handle* h, uint32_t n_sites, const int32_t* pos, const uint8_t* alt, uint32_t max_span) {
+    if (!h) return LVC_EINVAL;
+    if (n_sites && (!pos || !alt)) return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: null pos or alt");
+    if (n_sites > (1u << 20)) return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: %u sites, at most 2^20", n_sites);
+    if (n_sites && (max_span < 1 || max_span > 65535))
+        return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: max_span %u outside 1..65535", max_span);
+    CU(cudaSetDevice(h->device));
+    std::vector<uint8_t> ref;
+    if (n_sites) {
+        for (uint32_t k = 0; k < n_sites; ++k) {
+            if (pos[k] < 0 || pos[k] >= h->G)
+                return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: site %u at %d outside [0, %lld)", k, pos[k], (long long)h->G);
+            if (k && pos[k] <= pos[k - 1])
+                return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: positions not strictly ascending at site %u (%d after %d)", k,
+                            pos[k], pos[k - 1]);
+            if (!nibble_of(alt[k]) && alt[k] != '-')
+                return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: site %u at %d: alt 0x%02x is not A, C, G, T or '-'", k, pos[k],
+                            alt[k]);
+        }
+        // the reference letters at the sites
+        ref.resize((size_t)(pos[n_sites - 1] - pos[0]) + 1);
+        CU(cudaMemcpyAsync(ref.data(), h->d_ref + pos[0], ref.size(), cudaMemcpyDeviceToHost, h->stream));
+        CU(cudaStreamSynchronize(h->stream));
+    }
+    std::vector<LinkSite> site(n_sites);
+    std::vector<uint32_t> npart(n_sites, 0);
+    uint32_t window = 0;                         // most sites inside a window of max_span + 1 positions
+    for (uint32_t k = 0, a = 0; k < n_sites; ++k) {
+        const uint8_t rc = (uint8_t)toupper(ref[(size_t)(pos[k] - pos[0])]);
+        if (!nibble_of(rc))
+            return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: site %u at %d: reference letter '%c' is not A, C, G or T", k, pos[k],
+                        rc);
+        if (rc == alt[k])
+            return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: site %u at %d: alt '%c' equals the reference letter", k, pos[k], rc);
+        while ((int64_t)pos[k] - pos[a] > (int64_t)max_span) ++a;
+        window = std::max(window, k - a + 1);
+        if (window > kLinkMaxWindow)
+            return fail(h, LVC_EINVAL, "lvc_set_linkage_sites: %u sites inside the %u positions [%d, %d]; at most %u sites may lie "
+                        "inside any window of max_span + 1 positions", k - a + 1, max_span + 1, pos[k] - (int)max_span, pos[k],
+                        kLinkMaxWindow);
+        site[k] = LinkSite{0, nibble_of(rc), alt[k] == '-' ? kLinkDeletion : nibble_of(alt[k]), (uint8_t)(k - a), 0};
+        for (uint32_t x = a; x < k; ++x) ++npart[x];
+    }
+    uint64_t pairs = 0;
+    for (uint32_t k = 0; k < n_sites; ++k) { site[k].off = (uint32_t)pairs; pairs += npart[k]; }
+    CU(cudaStreamSynchronize(h->stream));
+    free_linkage(h);
+    if (!n_sites) return LVC_OK;
+    LinkTable t = {nullptr, nullptr, nullptr, n_sites};
+    int32_t* d_pos = nullptr;
+    LinkSite* d_site = nullptr;
+    if (cudaMalloc(&d_pos, n_sites * sizeof(int32_t)) != cudaSuccess || cudaMalloc(&d_site, n_sites * sizeof(LinkSite)) != cudaSuccess ||
+        cudaMalloc(&t.counts, std::max<uint64_t>(pairs, 1) * 9 * sizeof(uint32_t)) != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(d_pos); cudaFree(d_site);
+        return fail(h, LVC_ENOMEM, "lvc_set_linkage_sites: no device memory for %llu pairs (%llu bytes)", (unsigned long long)pairs,
+                    (unsigned long long)(pairs * 9 * sizeof(uint32_t)));
+    }
+    t.pos = d_pos; t.site = d_site;
+    h->link = t;
+    h->link_pairs = pairs;
+    h->link_pos.assign(pos, pos + n_sites);
+    h->link_alt.assign(alt, alt + n_sites);
+    h->link_npart = std::move(npart);
+    CU(cudaMemcpyAsync(d_pos, pos, n_sites * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_site, site.data(), n_sites * sizeof(LinkSite), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemsetAsync(t.counts, 0, std::max<uint64_t>(pairs, 1) * 9 * sizeof(uint32_t), h->stream));
+    CU(cudaStreamSynchronize(h->stream));     // `site` goes out of scope
+    return LVC_OK;
+}
+
+int lvc_copy_linkage(lvc_handle* h, lvc_linkage_pair* out, uint32_t cap, uint32_t* n_out) {
+    NvtxRange nvtx_range("lvc_copy_linkage");
+    if (!h || !n_out || (cap && !out)) return LVC_EINVAL;
+    if (!h->link.counts) return fail(h, LVC_EINVAL, "linkage counting is off (lvc_set_linkage_sites)");
+    *n_out = (uint32_t)h->link_pairs;
+    if (h->link_pairs > cap) return LVC_OK;
+    CU(cudaSetDevice(h->device));
+    std::vector<uint32_t> counts(h->link_pairs * 9);
+    if (h->link_pairs)
+        CU(cudaMemcpyAsync(counts.data(), h->link.counts, counts.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    size_t j = 0;
+    for (uint32_t a = 0; a < h->link.n_sites; ++a)
+        for (uint32_t b = a + 1; b <= a + h->link_npart[a]; ++b, ++j) {
+            lvc_linkage_pair& o = out[j];
+            o.pos_a = h->link_pos[a]; o.pos_b = h->link_pos[b];
+            o.alt_a = h->link_alt[a]; o.alt_b = h->link_alt[b];
+            o.pad = 0;
+            memcpy(o.count, counts.data() + j * 9, 9 * sizeof(uint32_t));
+        }
+    return LVC_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -64,6 +64,11 @@ assert C.sizeof(ConsensusStats) == 128
 INSERTION_DTYPE = np.dtype([("pos", "<i4"), ("len", "<u4"), ("seq", "<u8"), ("count", "<u4"), ("depth", "<u4")])
 assert INSERTION_DTYPE.itemsize == 24
 
+# lvc_linkage_pair (include/lvc.h): the two sites, their alts (ASCII) and count[state_a][state_b], REF 0 / ALT 1 / OTHER 2
+LINKAGE_DTYPE = np.dtype([("pos_a", "<i4"), ("pos_b", "<i4"), ("alt_a", "u1"), ("alt_b", "u1"), ("pad", "<u2"),
+                          ("count", "<u4", (3, 3))])
+assert LINKAGE_DTYPE.itemsize == 48
+
 _lib: Optional[C.CDLL] = None
 
 # every symbol include/lvc.h declares: (name, restype, argtypes)
@@ -118,6 +123,8 @@ SIGNATURES = [
     ("lvc_copy_insertions", C.c_int, [_H, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]),
     ("lvc_insertion_calls", C.c_int, [_H, C.c_int64, C.c_int64, C.c_uint64, C.c_double, C.c_void_p, C.c_uint32,
                                       C.POINTER(C.c_uint32)]),
+    ("lvc_set_linkage_sites", C.c_int, [_H, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32]),
+    ("lvc_copy_linkage", C.c_int, [_H, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]),
     ("lvc_num_planes", C.c_int, [_H]),
     ("lvc_plane_keys", C.c_int, [_H, C.c_void_p]),
     ("lvc_ensure_plane", C.c_int, [_H, C.c_uint16]),
@@ -607,6 +614,26 @@ class Handle:
             raise ValueError(f"min_depth must be >= 0, not {min_depth}")
         return self._insertion_query(lambda out, cap, n: self.lib.lvc_insertion_calls(
             self.h, int(p0), int(p1), int(min_depth), float(threshold), out, cap, n))
+
+    # ---- variant linkage
+    def set_linkage_sites(self, pos, alt, max_span: int):
+        """lvc_set_linkage_sites: count how the sites (pos[k], alt[k]) co-occur on reads from the next push on; clears
+        the counts.  `alt`: a str or bytes of 'A' 'C' 'G' 'T' '-', one per site.  No sites turns counting off."""
+        pos = np.ascontiguousarray(pos, dtype=np.int32)
+        alt = np.frombuffer(alt.encode("ascii") if isinstance(alt, str) else bytes(alt), dtype=np.uint8)
+        if pos.ndim != 1 or pos.size != alt.size:
+            raise ValueError(f"{pos.size} positions but {alt.size} alts")
+        self._check(self.lib.lvc_set_linkage_sites(self.h, pos.size, _ptr(pos), _ptr(alt), int(max_span)))
+
+    def copy_linkage(self) -> np.ndarray:
+        """lvc_copy_linkage: every pair (LINKAGE_DTYPE) in (a, b) order, zero counts included"""
+        cap, n = 0, C.c_uint32(0)
+        while True:
+            out = np.zeros(cap, dtype=LINKAGE_DTYPE)
+            self._check(self.lib.lvc_copy_linkage(self.h, _ptr(out) if cap else None, cap, C.byref(n)))
+            if n.value <= cap:
+                return out[:n.value]
+            cap = n.value
 
     # ---- tables
     def plane_keys(self) -> np.ndarray:

@@ -7,7 +7,7 @@ live_variant_caller.py:158-185 (record), :233-297 (VCF), utils.py:12-13 (to_phre
 from __future__ import annotations
 
 import math
-from typing import Dict, List, Sequence, Tuple
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -125,3 +125,18 @@ def splice_insertions(consensus: str, calls) -> str:
         last = p
     out.append(consensus[last:])
     return "".join(out)
+
+
+def linkage_r2(counts) -> Optional[float]:
+    """r^2 of two sites from the REF/ALT 2x2 of a linkage pair's 3x3 counts (count[state_a][state_b], REF 0, ALT 1):
+    n = n00 + n01 + n10 + n11, pa = (n10 + n11) / n, pb = (n01 + n11) / n, D = n11 / n - pa * pb,
+    r2 = D^2 / (pa (1 - pa) pb (1 - pb)); None when n == 0 or the denominator is 0"""
+    n00, n01, n10, n11 = (int(counts[a][b]) for a, b in ((0, 0), (0, 1), (1, 0), (1, 1)))
+    if n00 + n01 + n10 + n11 == 0:
+        return None
+    # the same in integers (D = (n00 n11 - n01 n10) / n^2, pa (1 - pa) = (n10 + n11)(n00 + n01) / n^2, ...), so that
+    # perfect linkage gives exactly 1.0
+    den = (n10 + n11) * (n00 + n01) * (n01 + n11) * (n00 + n10)
+    if den == 0:
+        return None
+    return (n00 * n11 - n01 * n10) ** 2 / den

@@ -222,6 +222,34 @@ class LiveVariantCaller:
         out["completeness"] = (n - st["n_N"]) / n
         return out
 
+    # ------------------------------------------------------------------ variant linkage (not in the reference API)
+    def track_linkage(self, sites, maxSpan: int = 300):
+        """Count, from now on, how the `sites` -- an iterable of (pos0, alt), pos0 0-based and ascending, alt one of
+        'A' 'C' 'G' 'T' or '-' for a deletion -- co-occur on the same reads (include/lvc.h lvc_set_linkage_sites): every two
+        sites at most maxSpan apart form a pair.  Call it before process_bam / process_batch: the counts cover the batches
+        pushed since, and calling it again starts them over; reset_memory and load_checkpoint clear them and keep the sites.
+        An empty list turns counting off."""
+        sites = [(int(p), str(a)) for p, a in sites]
+        with self._lock:
+            self._handle.set_linkage_sites([p for p, _ in sites], "".join(a for _, a in sites), int(maxSpan))
+
+    def linkage(self, minReads: int = 1) -> List[dict]:
+        """Every pair of tracked sites whose REF/ALT states were both seen on at least minReads reads, in (pos_a, pos_b)
+        order: {"pos_a", "alt_a", "pos_b", "alt_b", "counts": 3x3 list [state_a][state_b] (REF 0, ALT 1, OTHER 2),
+        "n": reads with REF or ALT at both sites, "r2": squared correlation of the ALT states on those reads, None when
+        n is 0 or a site does not vary}."""
+        with self._lock:
+            pairs = self._handle.copy_linkage()
+        out = []
+        for p in pairs:
+            counts = p["count"].tolist()
+            n = counts[0][0] + counts[0][1] + counts[1][0] + counts[1][1]
+            if n < minReads:
+                continue
+            out.append({"pos_a": int(p["pos_a"]), "alt_a": chr(p["alt_a"]), "pos_b": int(p["pos_b"]),
+                        "alt_b": chr(p["alt_b"]), "counts": counts, "n": n, "r2": records.linkage_r2(counts)})
+        return out
+
     # ------------------------------------------------------------------ state <-> reference schema
     def _export_tables(self):
         h = self._handle

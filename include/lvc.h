@@ -338,6 +338,49 @@ int lvc_copy_insertions(lvc_handle* h, lvc_insertion* out, uint32_t cap, uint32_
 int lvc_insertion_calls(lvc_handle* h, int64_t p0, int64_t p1, uint64_t min_depth, double threshold,
                         lvc_insertion* out, uint32_t cap, uint32_t* n_out);
 
+/* ---- variant linkage [EXT] ---------------------------------------------------------------------
+ * Whether variants sit on the same molecules: for registered sites, how their states co-occur on the same reads.  The count
+ * tables above keep no trace of which read carried which base, so this is counted while each batch is on the device.
+ * Opt-in: records, VCF, CSV, `memory`, checkpoints, the consensus and the insertion counts do not change, and while counting
+ * is on each push launches exactly one more kernel.
+ * Sites.  n_sites entries (pos[k], alt[k]): pos 0-based, strictly ascending, inside [0, G); alt one of 'A' 'C' 'G' 'T' '-'
+ * ('-' = a deletion); the reference letter at pos, upper-cased, must be A/C/G/T and differ from alt.  A pair is two sites
+ * a < b with pos_b - pos_a <= max_span (1..65535); the partners of a are the sites a+1 .. last(a), and pairs are numbered
+ * in (a, b) order.
+ * Which reads count: those the deposit walks (keep bit0 set, read_passes_filter, at least one reference-consuming op, inside
+ * [0, G)), as for insertions.  The mates of a pair are separate reads.
+ * State of a site on a read, from the read's pileup entry at pos (the entry the deposit adds to totalDepth):
+ *   absent   no entry (outside the aligned span, in a soft clip), or the entry fails the base-quality rule: for a base its
+ *            quality, for a deletion or ref-skip entry the quality htslib's resolve_cigar2 assigns to it (the query base at
+ *            the start of the op, 0 past the end of the read);
+ *   REF (0)  the base is the reference letter;
+ *   ALT (1)  the base is alt, or the entry is a deletion / ref-skip and alt is '-';
+ *   OTHER (2) anything else: another nibble code (N included), or a deletion / ref-skip when alt is a base.
+ * Qualities are read as the batch carries them (mate-overlap rewrites need no special case); every batch form counts the same
+ * values.  Counts: every pair whose two sites are both present on a read adds 1 to count[state_a][state_b], at most once
+ * per read.  They cover the batches pushed since the last lvc_set_linkage_sites or lvc_reset: setting sites clears them,
+ * lvc_reset clears them and keeps the sites; imports, checkpoints and lvc_reduce_tables do not touch them.  With read-chunk
+ * sharding or peer tables each handle counts the reads pushed to it; the chunks of the ranks are disjoint, so the sample's
+ * counts are the sum over the ranks (no exchange is made).
+ * lvc_set_linkage_sites  n_sites = 0 turns counting off and frees the tables (pos, alt and max_span are then ignored).
+ *                        LVC_EINVAL, with a message naming the number, for n_sites > 2^20, max_span outside 1..65535, more
+ *                        than 64 sites inside any window of max_span + 1 positions (this bounds the per-read state of the
+ *                        kernel, so no read is ever truncated; a dense panel can use a smaller span), unsorted or duplicate
+ *                        positions, a bad alt, alt equal to the reference letter, or a reference letter that is not A/C/G/T;
+ *                        LVC_ENOMEM if the pair table (36 bytes per pair) cannot be allocated.  A refused call keeps the
+ *                        previous sites and counts.
+ * lvc_copy_linkage       every pair in (a, b) order, zero counts included; *n_out = the number of pairs, and out is written
+ *                        only if it is <= cap (else call again with a larger buffer).  LVC_EINVAL while counting is off.
+ * Timer 5 of lvc_get_timing times the counting kernel. */
+typedef struct lvc_linkage_pair {
+    int32_t pos_a, pos_b;   /* 0-based positions of the two sites, pos_a < pos_b */
+    uint8_t alt_a, alt_b;   /* 'A' 'C' 'G' 'T' or '-' */
+    uint16_t pad;
+    uint32_t count[3][3];   /* [state_a][state_b]: REF 0, ALT 1, OTHER 2 */
+} lvc_linkage_pair;         /* 48 bytes */
+int lvc_set_linkage_sites(lvc_handle* h, uint32_t n_sites, const int32_t* pos, const uint8_t* alt, uint32_t max_span);
+int lvc_copy_linkage(lvc_handle* h, lvc_linkage_pair* out, uint32_t cap, uint32_t* n_out);
+
 /* ---- table access: self.memory (live_variant_caller.py:31), checkpoints (:40-52), tests, NCCL ----
  * A "plane" holds, for one (allele group, quality) key, uint32 counts [G][4].  key = group<<8 | q;
  * group 0 = A,C,G,T (slots 0..3); groups 1..3 hold the other BAM nibble codes:
@@ -416,7 +459,8 @@ uint64_t lvc_launch_count(lvc_handle* h);
 uint64_t lvc_h2d_payload_bytes(lvc_handle* h);
 /* per-kernel device time from CUDA events recorded on the handle's stream around every launch while
  * timing is on.  which: 0 = tiled deposit, 1 = general deposit, 2 = genotype, 3 = consensus, 4 = insertion counts (only
- * on a handle that counts them, lvc_enable_insertions).  Reading resets. */
+ * on a handle that counts them, lvc_enable_insertions), 5 = linkage counts (only with sites, lvc_set_linkage_sites).
+ * Reading resets. */
 int lvc_set_timing(lvc_handle* h, int on);
 int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launches);
 int lvc_version(void);
