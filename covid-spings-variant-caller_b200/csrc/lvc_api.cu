@@ -23,6 +23,7 @@
 #include "consensus.cuh"
 #include "insertions.cuh"
 #include "linkage.cuh"
+#include "strand.cuh"
 #include "deposit_select.hpp"
 #include "overlap.hpp"
 #include "qcode.hpp"
@@ -130,10 +131,15 @@ struct lvc_handle {
     std::vector<uint8_t> link_alt;
     std::vector<uint32_t> link_npart;        // partners after each site
 
+    // strand counts (lvc_enable_strand_counts): d_rev == nullptr while counting is off.  [kStrandRows][G]: the reverse-strand
+    // counts of the 16 allele slots, then of deletions.  Queries are gated by ins_uncovered, as the insertion counts are.
+    uint32_t* d_rev = nullptr;
+    DevBuf s_query;
+
     // optional per-kernel timing (CUDA events on the launching stream)
     bool timing = false;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[6];   // 0 tiled deposit, 1 general deposit, 2 genotype, 3 consensus,
-                                                              // 4 insertion counts, 5 linkage counts
+    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> ev[7];   // 0 tiled deposit, 1 general deposit, 2 genotype, 3 consensus,
+                                                              // 4 insertion counts, 5 linkage counts, 6 strand counts
     std::vector<cudaEvent_t> ev_pool;
 };
 
@@ -350,15 +356,16 @@ void lvc_destroy(lvc_handle* h) {
     cudaFree(h->d_first_arr); cudaFree(h->d_newkeys); cudaFree(h->d_replay); cudaFree(h->d_status); cudaFree(h->d_keymap);
     if (h->h_status) cudaFreeHost(h->h_status);
     if (h->h_sample) cudaFreeHost(h->h_sample);
-    for (int w = 0; w < 6; ++w) for (auto& pr : h->ev[w]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
+    for (int w = 0; w < 7; ++w) for (auto& pr : h->ev[w]) { cudaEventDestroy(pr.first); cudaEventDestroy(pr.second); }
     for (auto e : h->ev_pool) cudaEventDestroy(e);
     cudaFree(h->d_elut); cudaFree(h->d_out_depth); cudaFree(h->d_out_ad); cudaFree(h->d_out_lik);
     cudaFree(h->d_cand_count);
     cudaFree(h->ins.keys); cudaFree(h->ins.counts); cudaFree(h->ins.dropped);
     cudaFree((void*)h->link.pos); cudaFree((void*)h->link.site); cudaFree(h->link.counts);
+    cudaFree(h->d_rev);
     for (DevBuf* b : {&h->b_pos, &h->b_flag, &h->b_mapq, &h->b_keep, &h->b_coff, &h->b_cig, &h->b_soff, &h->b_seq,
                       &h->b_qual, &h->g_order_ptrs, &h->g_order_keys, &h->g_cand, &h->g_pconst, &h->c_order_ptrs,
-                      &h->c_seq, &h->c_stats, &h->i_list, &h->i_scratch})
+                      &h->c_seq, &h->c_stats, &h->i_list, &h->i_scratch, &h->s_query})
         cudaFree(b->p);
     if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
     delete h;
@@ -407,6 +414,7 @@ int lvc_reset(lvc_handle* h) {
         CU(cudaMemsetAsync(h->ins.dropped, 0, sizeof(uint32_t), h->stream));
     }
     if (h->link.counts) CU(cudaMemsetAsync(h->link.counts, 0, h->link_pairs * 9 * sizeof(uint32_t), h->stream));
+    if (h->d_rev) CU(cudaMemsetAsync(h->d_rev, 0, kStrandRows * G * sizeof(uint32_t), h->stream));
     h->tables_touched = false;
     h->ins_uncovered = false;
     h->ordinal = 0;
@@ -571,6 +579,19 @@ static int launch_count_linkage(lvc_handle* h, const BatchView& bv) {
     return LVC_OK;
 }
 
+// The reverse-strand counts of one batch (lvc_enable_strand_counts), launched like launch_count_insertions and behind the
+// linkage counts.
+static int launch_count_strands(lvc_handle* h, const BatchView& bv) {
+    if (!h->d_rev || bv.n_reads == 0) return LVC_OK;
+    StrandCountParams cp;
+    cp.G = h->G; cp.min_bq = h->min_bq; cp.min_mq = h->min_mq;
+    { KernelTimer t(h, 6);
+      CU(launch_kernel(h, k_count_strands, dim3((bv.n_reads + kStrandReads - 1) / kStrandReads), dim3(kStrandThreads), 0, true,
+                       bv, h->d_rev, cp, bv.n_reads)); }
+    CU(cudaGetLastError());
+    return LVC_OK;
+}
+
 static int deposit_with_replay(lvc_handle* h, const BatchView& bv, uint64_t n_cigar_ops, uint64_t n_qual,
                                const lvc_batch* account = nullptr) {
     if ((uint64_t)h->ordinal + bv.n_reads >= 0xFFFFFFFFull)
@@ -582,6 +603,8 @@ static int deposit_with_replay(lvc_handle* h, const BatchView& bv, uint64_t n_ci
     rc = launch_count_insertions(h, bv);           // once per batch: the replay pass below does not count again
     if (rc) return rc;
     rc = launch_count_linkage(h, bv);
+    if (rc) return rc;
+    rc = launch_count_strands(h, bv);
     if (rc) return rc;
     CU(cudaMemcpyAsync(h->h_status, h->d_status, ST_WORDS * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
     CU(cudaMemcpyAsync(h->h_status + ST_WORDS, h->d_newkeys, 32 * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
@@ -862,6 +885,8 @@ int lvc_push_batch_device_async(lvc_handle* h, const lvc_batch* b) {
     if (rc) return rc;
     rc = launch_count_linkage(h, bv);
     if (rc) return rc;
+    rc = launch_count_strands(h, bv);
+    if (rc) return rc;
     h->ordinal += b->n_reads;
     return LVC_OK;
 }
@@ -888,9 +913,10 @@ int lvc_set_timing(lvc_handle* h, int on) {
 }
 
 int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launches) {
-    if (!h || which < 0 || which > 5 || !ms_total || !n_launches) return LVC_EINVAL;
+    if (!h || which < 0 || which > 6 || !ms_total || !n_launches) return LVC_EINVAL;
     if (which == 4 && !h->ins.keys) return fail(h, LVC_EINVAL, "timer 4 (insertion counts) needs lvc_enable_insertions");
     if (which == 5 && !h->link.counts) return fail(h, LVC_EINVAL, "timer 5 (linkage counts) needs lvc_set_linkage_sites");
+    if (which == 6 && !h->d_rev) return fail(h, LVC_EINVAL, "timer 6 (strand counts) needs lvc_enable_strand_counts");
     CU(cudaSetDevice(h->device));
     CU(cudaStreamSynchronize(h->stream));
     double tot = 0.0;
@@ -1303,6 +1329,8 @@ static void free_linkage(lvc_handle* h) {
     h->link_pos.clear(); h->link_alt.clear(); h->link_npart.clear();
 }
 
+static const char kNibbleLetters[] = "=ACMGRSVTWYHKDBN";       // htslib seq_nt16_str: letter index = BAM nibble
+
 static uint8_t nibble_of(uint8_t c) {
     switch (c) { case 'A': return 1; case 'C': return 2; case 'G': return 4; case 'T': return 8; default: return 0; }
 }
@@ -1398,6 +1426,73 @@ int lvc_copy_linkage(lvc_handle* h, lvc_linkage_pair* out, uint32_t cap, uint32_
             o.pad = 0;
             memcpy(o.count, counts.data() + j * 9, 9 * sizeof(uint32_t));
         }
+    return LVC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// strand counts
+// ------------------------------------------------------------------------------------------------
+int lvc_enable_strand_counts(lvc_handle* h) {
+    if (!h) return LVC_EINVAL;
+    if (h->G > 0x7FFFFFFF) return fail(h, LVC_EINVAL, "lvc_enable_strand_counts: contig longer than 2^31 - 1");
+    if (h->peer_ranks > 1) return fail(h, LVC_EINVAL, "lvc_enable_strand_counts: refused on a handle with peer tables attached");
+    if (h->tables_touched)
+        return fail(h, LVC_EINVAL, "lvc_enable_strand_counts: the tables already hold counts; call it after lvc_create or lvc_reset");
+    if (h->d_rev) return LVC_OK;
+    CU(cudaSetDevice(h->device));
+    const size_t bytes = (size_t)kStrandRows * (size_t)h->G * sizeof(uint32_t);
+    if (cudaMalloc(&h->d_rev, bytes) != cudaSuccess) {
+        cudaGetLastError();
+        h->d_rev = nullptr;
+        return fail(h, LVC_ENOMEM, "lvc_enable_strand_counts: no device memory for %zu bytes", bytes);
+    }
+    CU(cudaMemsetAsync(h->d_rev, 0, bytes, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    return LVC_OK;
+}
+
+int lvc_strand_counts(lvc_handle* h, uint32_t n, const int32_t* pos, const uint8_t* allele, uint32_t* fwd, uint32_t* rev) {
+    NvtxRange nvtx_range("lvc_strand_counts");
+    if (!h) return LVC_EINVAL;
+    if (n && (!pos || !allele || !fwd || !rev)) return fail(h, LVC_EINVAL, "lvc_strand_counts: null array");
+    if (!h->d_rev) return fail(h, LVC_EINVAL, "strand counting is off (lvc_enable_strand_counts)");
+    if (h->ins_uncovered)
+        return fail(h, LVC_EINVAL, "the tables hold imported or reduced counts that the strand counts do not cover; "
+                    "lvc_reset starts over");
+    // the table row of each query: the allele slot of its nibble letter, 16 for '-'
+    std::vector<uint8_t> row(n);
+    for (uint32_t k = 0; k < n; ++k) {
+        if (pos[k] < 0 || pos[k] >= h->G)
+            return fail(h, LVC_EINVAL, "lvc_strand_counts: query %u at %d outside [0, %lld)", k, pos[k], (long long)h->G);
+        const char* nib = allele[k] ? strchr(kNibbleLetters, toupper(allele[k])) : nullptr;
+        if (allele[k] == '-') row[k] = 16;
+        else if (nib) row[k] = (uint8_t)nibble_gs((uint32_t)(nib - kNibbleLetters));
+        else return fail(h, LVC_EINVAL, "lvc_strand_counts: query %u: allele 0x%02x is not a nibble letter (=ACMGRSVTWYHKDBN) or '-'",
+                         k, allele[k]);
+    }
+    if (n == 0) return LVC_OK;
+    CU(cudaSetDevice(h->device));
+    int rc = upload_consensus_planes(h);
+    if (rc) return rc;
+    // device scratch: pos [n], then fwd [n], rev [n], then the rows [n]
+    rc = ensure(h, h->s_query, (size_t)n * 13);
+    if (rc) return rc;
+    int32_t* d_pos = (int32_t*)h->s_query.p;
+    uint32_t* d_fwd = (uint32_t*)(d_pos + n);
+    uint32_t* d_rv = d_fwd + n;
+    uint8_t* d_row = (uint8_t*)(d_rv + n);
+    CU(cudaMemcpyAsync(d_pos, pos, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(d_row, row.data(), n, cudaMemcpyHostToDevice, h->stream));
+    StrandQueryParams qp;
+    qp.G = h->G;
+    for (int g = 0; g < 5; ++g) qp.grp_begin[g] = h->cons_grp_begin[g];
+    CU(launch_kernel(h, k_strand_query, dim3((n + kStrandQueryThreads - 1) / kStrandQueryThreads), dim3(kStrandQueryThreads), 0,
+                     false, qp, (const uint32_t* const*)h->c_order_ptrs.p, (const uint32_t*)h->d_dels, (const uint32_t*)h->d_rev,
+                     (const int32_t*)d_pos, (const uint8_t*)d_row, d_fwd, d_rv, n));
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(fwd, d_fwd, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(rev, d_rv, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));     // `row` goes out of scope
     return LVC_OK;
 }
 

@@ -87,6 +87,7 @@ int lvc_peer_detach(lvc_handle* h) {
 int lvc_peer_attach(lvc_handle* h, int rank, int n_ranks, const void* const* blobs, const size_t* lens) {
     if (!h || !blobs || !lens || n_ranks < 1 || n_ranks > kMaxPeers || rank < 0 || rank >= n_ranks) return LVC_EINVAL;
     if (h->ins.keys) return fail(h, LVC_EINVAL, "lvc_peer_attach: refused on a handle that counts insertions");
+    if (h->d_rev) return fail(h, LVC_EINVAL, "lvc_peer_attach: refused on a handle that counts strands");
     int rc = lvc_peer_detach(h);
     if (rc) return rc;
     if (n_ranks == 1) return LVC_OK;

@@ -125,6 +125,8 @@ SIGNATURES = [
                                       C.POINTER(C.c_uint32)]),
     ("lvc_set_linkage_sites", C.c_int, [_H, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32]),
     ("lvc_copy_linkage", C.c_int, [_H, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint32)]),
+    ("lvc_enable_strand_counts", C.c_int, [_H]),
+    ("lvc_strand_counts", C.c_int, [_H, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     ("lvc_num_planes", C.c_int, [_H]),
     ("lvc_plane_keys", C.c_int, [_H, C.c_void_p]),
     ("lvc_ensure_plane", C.c_int, [_H, C.c_uint16]),
@@ -634,6 +636,23 @@ class Handle:
             if n.value <= cap:
                 return out[:n.value]
             cap = n.value
+
+    # ---- strand counts
+    def enable_strand_counts(self):
+        """lvc_enable_strand_counts: count reverse-strand pileup entries from the next push on (only on empty tables)"""
+        self._check(self.lib.lvc_enable_strand_counts(self.h))
+
+    def strand_counts(self, pos, allele):
+        """lvc_strand_counts: (fwd, rev) uint32 arrays, the forward and reverse entries of allele[k] at pos[k].  `allele`:
+        a str or bytes of nibble letters (=ACMGRSVTWYHKDBN, either case) or '-' for deletions, one per position."""
+        pos = np.ascontiguousarray(pos, dtype=np.int32).reshape(-1)
+        allele = np.frombuffer(allele.encode("ascii") if isinstance(allele, str) else bytes(allele), dtype=np.uint8)
+        if pos.size != allele.size:
+            raise ValueError(f"{pos.size} positions but {allele.size} alleles")
+        fwd = np.zeros(pos.size, dtype=np.uint32)
+        rev = np.zeros(pos.size, dtype=np.uint32)
+        self._check(self.lib.lvc_strand_counts(self.h, pos.size, _ptr(pos), _ptr(allele), _ptr(fwd), _ptr(rev)))
+        return fwd, rev
 
     # ---- tables
     def plane_keys(self) -> np.ndarray:

@@ -69,23 +69,106 @@ VCF_INFO_META = [
 ]
 
 
-def format_vcf(variants: List[dict], contigs: Sequence[Tuple[str, int]]) -> str:
+# the INFO metas write_vcf(strandBias=True) adds after VCF_INFO_META
+VCF_STRAND_META = [
+    ("DP4", "4", "Integer", "Reference-forward, reference-reverse, alternate-forward and alternate-reverse entries counted "
+                            "in DP"),
+    ("FS", "1", "Float", "Phred-scaled p-value of the two-sided Fisher exact test on the DP4 table (strand bias)"),
+    ("SOR", "1", "Float", "Symmetric odds ratio of the DP4 table with pseudocounts of 1 (strand bias)"),
+]
+
+
+def format_vcf(variants: List[dict], contigs: Sequence[Tuple[str, int]], strand: Optional[List[dict]] = None) -> str:
     """VCF 4.2 text the way pysam/htslib writes the reference's records (live_variant_caller.py:235-295):
     INFO metas DP, AD, GL, PL, SCORE; one ##contig per FASTA contig; records stably sorted by
-    (start, SCORE); CHROM = first header contig (new_record is called without a contig)."""
+    (start, SCORE); CHROM = first header contig (new_record is called without a contig).
+    `strand`: the strand_bias rows of `variants`, in their order.  With them the header gains the VCF_STRAND_META lines and
+    the INFO of every record with counts gains DP4, FS and SOR (3 decimals); without them the text is unchanged."""
     lines = ["##fileformat=VCFv4.2", '##FILTER=<ID=PASS,Description="All filters passed">']
     for vid, typ, desc in VCF_INFO_META:
         lines.append(f'##INFO=<ID={vid},Number=1,Type={typ},Description="{desc}">')
+    if strand is not None:
+        if len(strand) != len(variants):
+            raise ValueError(f"{len(strand)} strand rows for {len(variants)} records")
+        for vid, num, typ, desc in VCF_STRAND_META:
+            lines.append(f'##INFO=<ID={vid},Number={num},Type={typ},Description="{desc}">')
     for name, length in contigs:
         lines.append(f"##contig=<ID={name},length={length}>")
     lines.append("#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO")
     chrom = contigs[0][0]
-    for v in sorted(variants, key=lambda v: (v["start"], v["info"]["SCORE"])):
+    order = sorted(range(len(variants)), key=lambda k: (variants[k]["start"], variants[k]["info"]["SCORE"]))
+    for k in order:
+        v = variants[k]
         i = v["info"]
-        lines.append(f'{chrom}\t{v["start"] + 1}\t.\t{v["alleles"][0]}\t{v["alleles"][1]}\t{fmt_g_float32(v["qual"])}'
-                     f'\t.\tDP={i["DP"]};AD={i["AD"]};GL={fmt_g_float32(i["GL"])};PL={i["PL"]};'
-                     f'SCORE={fmt_g_float32(i["SCORE"])}')
+        line = (f'{chrom}\t{v["start"] + 1}\t.\t{v["alleles"][0]}\t{v["alleles"][1]}\t{fmt_g_float32(v["qual"])}'
+                f'\t.\tDP={i["DP"]};AD={i["AD"]};GL={fmt_g_float32(i["GL"])};PL={i["PL"]};'
+                f'SCORE={fmt_g_float32(i["SCORE"])}')
+        if strand is not None and strand[k]["ref_fwd"] is not None:
+            sb = strand[k]
+            line += (f';DP4={sb["ref_fwd"]},{sb["ref_rev"]},{sb["alt_fwd"]},{sb["alt_rev"]}'
+                     f';FS={sb["fs"]:.3f};SOR={sb["sor"]:.3f}')
+        lines.append(line)
     return "\n".join(lines) + "\n"
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# strand bias
+# ---------------------------------------------------------------------------------------------------------------------
+_LN10 = math.log(10.0)
+
+
+def _log_choose(n: int, k: int) -> float:
+    return math.lgamma(n + 1) - math.lgamma(k + 1) - math.lgamma(n - k + 1)
+
+
+def fisher_log_p(ref_fwd: int, ref_rev: int, alt_fwd: int, alt_rev: int) -> float:
+    """natural log of the two-sided Fisher exact p-value of the 2x2 table [[ref_fwd, ref_rev], [alt_fwd, alt_rev]]: the sum
+    of the hypergeometric probabilities (margins fixed) that are <= the observed one x (1 + 1e-7), at most 1.  Computed in
+    log space, so tables of tens of thousands of reads do not underflow."""
+    a, b, c, d = int(ref_fwd), int(ref_rev), int(alt_fwd), int(alt_rev)
+    r1, r2, c1 = a + b, c + d, a + c
+    n = r1 + r2
+    lo, hi = max(0, c1 - r2), min(r1, c1)
+    base = -_log_choose(n, c1)
+
+    def lp(x):
+        return _log_choose(r1, x) + _log_choose(r2, c1 - x) + base
+
+    cut = lp(a) + math.log1p(1e-7)
+    terms = [t for t in (lp(x) for x in range(lo, hi + 1)) if t <= cut]
+    m = max(terms)
+    return min(0.0, m + math.log(sum(math.exp(t - m) for t in terms)))
+
+
+def fisher_p(ref_fwd: int, ref_rev: int, alt_fwd: int, alt_rev: int) -> float:
+    """two-sided Fisher exact p-value (fisher_log_p); 0.0 where it is below the smallest double"""
+    return math.exp(fisher_log_p(ref_fwd, ref_rev, alt_fwd, alt_rev))
+
+
+def fisher_strand(ref_fwd: int, ref_rev: int, alt_fwd: int, alt_rev: int) -> float:
+    """FS = -10 log10(fisher_p), from the log p-value (finite for any counts)"""
+    return -10.0 * fisher_log_p(ref_fwd, ref_rev, alt_fwd, alt_rev) / _LN10 + 0.0
+
+
+def strand_odds_ratio(ref_fwd: int, ref_rev: int, alt_fwd: int, alt_rev: int) -> float:
+    """GATK's StrandOddsRatio: with t00, t01, t10, t11 = ref_fwd, ref_rev, alt_fwd, alt_rev each + 1 and
+    R = (t00 t11) / (t01 t10), SOR = ln(R + 1/R) + ln(min(t00, t01) / max(t00, t01)) - ln(min(t10, t11) / max(t10, t11))"""
+    t00, t01, t10, t11 = int(ref_fwd) + 1, int(ref_rev) + 1, int(alt_fwd) + 1, int(alt_rev) + 1
+    r = (t00 * t11) / (t01 * t10)
+    return math.log(r + 1.0 / r) + math.log(min(t00, t01) / max(t00, t01)) - math.log(min(t10, t11) / max(t10, t11))
+
+
+def strand_row(v: dict, counts: Optional[Tuple[int, int, int, int]]) -> dict:
+    """one row of LiveVariantCaller.strand_bias: the record's start and alleles, its DP4 counts and the statistics (all
+    None without counts)"""
+    row = {"start": v["start"], "alleles": v["alleles"]}
+    if counts is None:
+        row.update(ref_fwd=None, ref_rev=None, alt_fwd=None, alt_rev=None, fisher_p=None, fs=None, sor=None)
+        return row
+    rf, rr, af, ar = (int(x) for x in counts)
+    row.update(ref_fwd=rf, ref_rev=rr, alt_fwd=af, alt_rev=ar, fisher_p=fisher_p(rf, rr, af, ar),
+               fs=fisher_strand(rf, rr, af, ar), sor=strand_odds_ratio(rf, rr, af, ar))
+    return row
 
 
 def format_site_csv(depth: np.ndarray, ad: np.ndarray, ref: str) -> str:

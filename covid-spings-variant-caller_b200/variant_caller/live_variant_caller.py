@@ -59,7 +59,7 @@ class LiveVariantCaller:
     def __init__(self, referenceFasta: str, minBaseQuality: int, minMappingQuality: int, minTotalDepth: int,
                  minAlleleDepth: int, minEvidenceRatio: float, maxVariants: int, device: Optional[int] = None,
                  maxDepth: int = capi.MAX_DEPTH_DEFAULT, ignoreOverlaps: bool = True, overlapModel: Optional[str] = None,
-                 countInsertions: bool = False, maxInsertionKeys: int = 1 << 20):
+                 countInsertions: bool = False, maxInsertionKeys: int = 1 << 20, countStrands: bool = False):
         self.minBaseQuality = minBaseQuality
         self.minMappingQuality = minMappingQuality
         self.minTotalDepth = minTotalDepth
@@ -74,6 +74,9 @@ class LiveVariantCaller:
         # maxInsertionKeys keys; records, VCF, memory and checkpoints never contain insertions
         self.countInsertions = bool(countInsertions)
         self.maxInsertionKeys = int(maxInsertionKeys)
+        # reverse-strand counts for strand_bias() and write_vcf(strandBias=True) (include/lvc.h lvc_enable_strand_counts):
+        # 17 x 4 bytes per reference position on the device; nothing else changes
+        self.countStrands = bool(countStrands)
         self.fastaFile = samio.Fasta(referenceFasta)
         self._device = _default_device() if device is None else device
         self._lock = threading.RLock()                      # the reference's callers use bare threads
@@ -96,6 +99,8 @@ class LiveVariantCaller:
                                    int(self.minMappingQuality), self._device)
         if self.countInsertions:
             self._handle.enable_insertions(self.maxInsertionKeys)
+        if self.countStrands:
+            self._handle.enable_strand_counts()
 
     def close(self):
         with self._lock:
@@ -155,11 +160,13 @@ class LiveVariantCaller:
                 out.setdefault(int(c["pos"]), {})[NIBBLE_CHARS[int(c["code"])]] = float(c["L"])
             return out
 
-    def write_vcf(self, outputVfc: str):
-        """live_variant_caller.py:233-297."""
+    def write_vcf(self, outputVfc: str, strandBias: bool = False):
+        """live_variant_caller.py:233-297.  strandBias=True (needs countStrands=True) adds DP4, FS and SOR to every record's
+        INFO and their three ##INFO lines to the header (strand_bias); without it the text is the reference's."""
         with self._lock:
             contigs = [(r, self.fastaFile.get_reference_length(r)) for r in self.fastaFile.references]
-            text = records.format_vcf(self.prepare_variants(), contigs)
+            variants = self.prepare_variants()
+            text = records.format_vcf(variants, contigs, self.strand_bias(variants) if strandBias else None)
         with open(outputVfc, "w") as fh:
             fh.write(text)
 
@@ -221,6 +228,27 @@ class LiveVariantCaller:
         out["breadth"] = {x: c / n for x, c in zip(depths, st["depth_ge"])}
         out["completeness"] = (n - st["n_N"]) / n
         return out
+
+    # ------------------------------------------------------------------ strand bias (not in the reference API)
+    def strand_bias(self, variants: Optional[List[Variant]] = None) -> List[dict]:
+        """Strand bias of each record of `variants` (default: prepare_variants()), in their order: {"start", "alleles",
+        "ref_fwd", "ref_rev", "alt_fwd", "alt_rev": the forward / reverse pileup entries of the REF and ALT letters at the
+        position, counted as DP counts them (bcftools DP4), "fisher_p": two-sided Fisher exact p-value of that 2x2 table,
+        "fs": -10 log10(fisher_p) (GATK FS), "sor": GATK's symmetric odds ratio (SOR)}.  Counts and statistics are None for
+        a record whose REF letter is not a nibble code.  Needs countStrands=True; after load_checkpoint it raises
+        (capi.LvcError) until reset_memory: the strand counts do not cover loaded tables."""
+        if not self.countStrands:
+            raise ValueError("this LiveVariantCaller does not count strands: construct it with countStrands=True")
+        with self._lock:
+            if variants is None:
+                variants = self.prepare_variants()
+            asked = [k for k, v in enumerate(variants)
+                     if all(len(a) == 1 and a.upper() in NIBBLE_CHARS for a in v["alleles"][:2])]
+            pos = [variants[k]["start"] for k in asked for _ in (0, 1)]
+            letters = "".join(variants[k]["alleles"][0] + variants[k]["alleles"][1] for k in asked)
+            fwd, rev = self._handle.strand_counts(pos, letters)
+        counts = {k: (fwd[2 * j], rev[2 * j], fwd[2 * j + 1], rev[2 * j + 1]) for j, k in enumerate(asked)}
+        return [records.strand_row(v, counts.get(k)) for k, v in enumerate(variants)]
 
     # ------------------------------------------------------------------ variant linkage (not in the reference API)
     def track_linkage(self, sites, maxSpan: int = 300):

@@ -381,6 +381,35 @@ typedef struct lvc_linkage_pair {
 int lvc_set_linkage_sites(lvc_handle* h, uint32_t n_sites, const int32_t* pos, const uint8_t* alt, uint32_t max_span);
 int lvc_copy_linkage(lvc_handle* h, lvc_linkage_pair* out, uint32_t cap, uint32_t* n_out);
 
+/* ---- strand counts [EXT] ----------------------------------------------------------------------------
+ * Strand bias of the evidence (bcftools DP4, GATK FS / SOR): how many of an allele's pileup entries came from forward and
+ * from reverse reads.  The count tables above hold no strand, and the reads are on the device only while their batch is
+ * deposited, so the reverse-strand share is counted then.  Opt-in: records, VCF, CSV, `memory`, checkpoints, the consensus
+ * and the insertion and linkage counts do not change, and while counting is on each push launches exactly one more kernel.
+ * Rule.  A handle that counts strands keeps rev[slot][p] for the 16 allele slots of the planes (group 0..3 x slot 0..3,
+ * the BAM nibble codes as in the plane keys below) and rev_del[p].  A read counts when
+ *   - the deposit walks it (keep bit0 set, read_passes_filter, at least one reference-consuming op, inside [0, G)),
+ *   - its flag has 0x10 (reverse strand) set,
+ *   - it has a pileup entry at p that the deposit adds to totalDepth;
+ * such a read adds 1 to rev[slot(nibble)][p] for a base, or to rev_del[p] for a deletion or ref-skip entry.  The quality
+ * rules are the deposit's: a base passes with its own quality; a deletion or ref-skip entry with the quality htslib's
+ * resolve_cigar2 assigns to it (the query base at the start of the op, 0 past the end of the read).  The mates of a pair
+ * count on their own strands; qualities are read as the batch carries them (mate-overlap rewrites need no special case);
+ * every batch form counts the same values.  The forward count is the sum of the allele's planes minus rev (dels minus
+ * rev_del for deletions), exactly, since both come from the same pushes.  Memory: 17 x 4 bytes x G.
+ * lvc_enable_strand_counts  only on empty tables (after lvc_create or lvc_reset), else LVC_EINVAL; LVC_EINVAL with peer
+ *                           tables attached (and lvc_peer_attach is refused on a handle that counts strands); LVC_EINVAL
+ *                           for G > 2^31 - 1; LVC_ENOMEM if the table cannot be allocated.  Calling it again is a no-op.
+ * lvc_strand_counts         n queries (pos[k], allele[k]): allele a nibble letter of "=ACMGRSVTWYHKDBN" (either case) or
+ *                           '-' for deletion and ref-skip entries; fwd[k] and rev[k] receive the allele's forward and
+ *                           reverse entries at pos[k].  LVC_EINVAL while counting is off, for a position outside [0, G) or
+ *                           an unknown letter, and after an import (so after loading a checkpoint) or lvc_reduce_tables
+ *                           until lvc_reset: the strand counts do not cover such tables.  lvc_reset clears the counts and
+ *                           keeps counting on.
+ * Timer 6 of lvc_get_timing times the counting kernel. */
+int lvc_enable_strand_counts(lvc_handle* h);
+int lvc_strand_counts(lvc_handle* h, uint32_t n, const int32_t* pos, const uint8_t* allele, uint32_t* fwd, uint32_t* rev);
+
 /* ---- table access: self.memory (live_variant_caller.py:31), checkpoints (:40-52), tests, NCCL ----
  * A "plane" holds, for one (allele group, quality) key, uint32 counts [G][4].  key = group<<8 | q;
  * group 0 = A,C,G,T (slots 0..3); groups 1..3 hold the other BAM nibble codes:
@@ -459,8 +488,8 @@ uint64_t lvc_launch_count(lvc_handle* h);
 uint64_t lvc_h2d_payload_bytes(lvc_handle* h);
 /* per-kernel device time from CUDA events recorded on the handle's stream around every launch while
  * timing is on.  which: 0 = tiled deposit, 1 = general deposit, 2 = genotype, 3 = consensus, 4 = insertion counts (only
- * on a handle that counts them, lvc_enable_insertions), 5 = linkage counts (only with sites, lvc_set_linkage_sites).
- * Reading resets. */
+ * on a handle that counts them, lvc_enable_insertions), 5 = linkage counts (only with sites, lvc_set_linkage_sites),
+ * 6 = strand counts (only on a handle that counts them, lvc_enable_strand_counts).  Reading resets. */
 int lvc_set_timing(lvc_handle* h, int on);
 int lvc_get_timing(lvc_handle* h, int which, double* ms_total, uint64_t* n_launches);
 int lvc_version(void);
